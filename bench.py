@@ -2,6 +2,7 @@
 """bench.py -- env-steps/s of the batched Walker3DCustomEnv-v0 hot path (BASELINE.json configs[1]).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--envs E] [--actions random|pd] [--impl reference]
+                  [--dump-outputs DIR]
 
 One "step" = one fused kernel launch stepping E envs per GPU through one control step (4 Bullet substeps +
 obs/reward/done/auto-reset).  Prints ONE JSON line (rank 0).  See DESIGN.md section "Measurement".
@@ -16,6 +17,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the source tree as it found it (it may be read-only)
 
 WORKLOAD = "Walker3DCustomEnv-v0 batched 16384 envs/GPU, flat ground"
 METRIC = "env-steps/sec (Walker3DCustomEnv-v0, 16384 envs/GPU, random actions)"
@@ -231,7 +233,7 @@ def main():
     _quiet_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=2000)
+    ap.add_argument("--steps", type=int, default=2000, help="timed steps of every measured loop")
     ap.add_argument("--warmup", type=int, default=200)
     ap.add_argument("--envs", type=int, default=16384, help="envs per GPU")
     ap.add_argument("--actions", default="random", choices=["random", "pd"])
@@ -246,7 +248,12 @@ def main():
                          "that the default headline run appends under \"also\"")
     ap.add_argument("--self-collision", type=int, default=1, choices=[0, 1],
                     help="1 = the reference's URDF_USE_SELF_COLLISION flags (robots.py:259-264); 0 = ablation")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the run, write what the last timed step of the headline workload returned (rank 0's "
+                         "envs) as DIR/<name>.npy, so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the CUDA path (--impl b200)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -297,17 +304,18 @@ def main():
     torch.cuda.set_device(dev)
     N, K, W = args.envs, args.steps, max(args.warmup, 3)
     ctx = dict(np=np, torch=torch, _lib=_lib, dist=dist, dev=dev, rank=rank, world=world, local_rank=local_rank)
-    line = measure(ctx, args.env, N, K, W, args.actions, args.self_collision)
+    outputs = {} if args.dump_outputs else None
+    line = measure(ctx, args.env, N, K, W, args.actions, args.self_collision, outputs)
     if args.also and args.env == "custom" and args.actions == "random" and args.self_collision:
         # BASELINE configs 2-5 next to the headline, every default run (so the 1/2/4/8-GPU scaling runs carry them):
-        # short device + e2e measurements with their own roofline fractions
+        # device + e2e measurements with their own roofline fractions
         also = {}
-        Ka, Wa = max(200, min(K, 400)), 20
+        Wa = 20
         for name, kind, n_envs, acts in (("walker3d_custom_pd", "custom", N, "pd"),
                                          ("walker3d_stepper", "stepper", N, "random"),
                                          ("monkey3d", "monkey", N, "random"),
                                          ("cassie_8192", "cassie", min(N, 8192), "random")):
-            r = measure(ctx, kind, n_envs, Ka, Wa, acts, 1)
+            r = measure(ctx, kind, n_envs, K, Wa, acts, 1)
             if r is not None:
                 also[name] = {k: r[k] for k in ("metric", "value", "unit", "ms_per_step", "steps", "warmup", "roofline",
                                                 "e2e", "gpu_launches", "episodes")}
@@ -318,6 +326,8 @@ def main():
         if dist:
             dist.destroy_process_group()
         return
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     if not args.no_cpu_baseline:
         ce = 256 if args.env == "cassie" else 2048
         v, dt, ks = cpu_reference_run(ce, 2000, 2, cores, time_budget=15.0, kind=args.env)
@@ -329,11 +339,29 @@ def main():
         dist.destroy_process_group()
 
 
+DUMP_BYTES = 64 << 20
 
 
-def measure(ctx, env_kind, N, K, W, actions, self_collision):
+def dump_outputs(out_dir, outputs):
+    """Write `outputs` (arrays with one row per env) as <out_dir>/<name>.npy in float32, and env_index.npy (float64):
+    the envs whose rows were written.  That is every env unless the files would exceed DUMP_BYTES; then it is a fixed,
+    seeded sample of them, the same from run to run."""
+    import numpy as np
+
+    n = len(outputs["obs"])
+    row_bytes = 8 + sum(4 * (a.size // n) for a in outputs.values())
+    keep = min(n, (DUMP_BYTES - 4096) // row_bytes)  # 4 KiB for the .npy headers
+    idx = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "env_index.npy"), idx.astype(np.float64))
+    for name, a in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a[idx], dtype=np.float32))
+
+
+def measure(ctx, env_kind, N, K, W, actions, self_collision, outputs=None):
     """One workload: W warm-up steps, K device-timed steps (CUDA events, L2 flushed in between, max over ranks) and the
-    host-buffer e2e leg.  Returns the JSON line (rank 0) or None."""
+    host-buffer e2e leg over K steps.  Returns the JSON line (rank 0) or None.  `outputs`, when given, receives as
+    NumPy arrays what the last timed step returned: obs, reward, done and truncated."""
     np, torch, _lib, dist, dev = ctx["np"], ctx["torch"], ctx["_lib"], ctx["dist"], ctx["dev"]
     rank, world, local_rank = ctx["rank"], ctx["world"], ctx["local_rank"]
     from mocca_envs_b200.distributed import shard_seed
@@ -415,6 +443,9 @@ def measure(ctx, env_kind, N, K, W, actions, self_collision):
         dist.barrier()
     torch.cuda.synchronize(dev)
     wall = time.perf_counter() - wall0
+    if outputs is not None:  # copied now: the e2e leg below steps the same env again
+        outputs.update((k, v.float().cpu().numpy()) for k, v in (
+            ("obs", obs), ("reward", rew), ("done", done), ("truncated", info["TimeLimit.truncated"])))
     launches = env.launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
     step_ms = [a.elapsed_time(b) for a, b in evs]
@@ -435,7 +466,6 @@ def measure(ctx, env_kind, N, K, W, actions, self_collision):
     episodes, ret_sum, len_sum, nonfinite, overflow, rows_all, conts_all = [float(x) for x in stat_vec.tolist()]
 
     # ---- e2e: same step through the host-buffer C-ABI entry point (pinned host memory, H2D + D2H in the timed region)
-    Ke = max(10, min(K, 100))
     # the same action stream as the device-timed loop, held in pinned host memory (a constant action per env would
     # be a different workload: joints pinned at their limits, more constraint rows)
     h_pool = act_pool.cpu().pin_memory()
@@ -451,14 +481,14 @@ def measure(ctx, env_kind, N, K, W, actions, self_collision):
         dist.barrier()
     torch.cuda.synchronize(dev)
     t0 = time.perf_counter()
-    for i in range(Ke):
+    for i in range(K):
         env.step_host(h_pool_np[(W + i) % pool], outs)  # returns once the D2H copies have completed
     torch.cuda.synchronize(dev)
     e2e_s = time.perf_counter() - t0
     te = torch.tensor([e2e_s], device=dev, dtype=torch.float64)
     if dist:
         dist.all_reduce(te, op=dist.ReduceOp.MAX)
-    e2e_value = N * world * Ke / float(te.item())
+    e2e_value = N * world * K / float(te.item())
     h2d = N * A * 4
     d2h = N * (env.obs_dim * 4 + 4 + 1 + 1)
 
@@ -537,7 +567,7 @@ def measure(ctx, env_kind, N, K, W, actions, self_collision):
                              "bytes_per_env_step": B_step,
                              "peak_source": "MEASURED_PEAKS.json" if peaks else "fallback"}},
         "e2e": {"value": e2e_value, "unit": "env-steps/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
-                "steps": Ke, "api": "mb200_step_host (pinned host buffers, returns when the D2H copies have landed)",
+                "steps": K, "api": "mb200_step_host (pinned host buffers, returns when the D2H copies have landed)",
                 "actions": "the device loop's random pool, read from pinned host memory"},
         "gpu_launches": int(launches),
         "clocks": clocks,
