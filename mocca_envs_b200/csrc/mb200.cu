@@ -732,7 +732,7 @@ int mb200_stats(mb200_env* e, double out[8], int reset) {
   CUDA_OK(cudaDeviceSynchronize());
   CUDA_OK(cudaMemcpy(&s, e->stats, sizeof(s), cudaMemcpyDeviceToHost));
   out[0] = (double)s.episodes; out[1] = s.ret_sum; out[2] = s.len_sum; out[3] = (double)s.nonfinite;
-  out[4] = (double)s.overflow; out[5] = (double)s.steps; out[6] = out[7] = 0.0;
+  out[4] = (double)s.overflow; out[5] = (double)s.steps_reached_sum; out[6] = out[7] = 0.0;
   if (reset) CUDA_OK(cudaMemset(e->stats, 0, sizeof(MbStats)));
   return 0;
 }

@@ -70,12 +70,28 @@ enum {  // Walker3DStepperEnv additions (env_locomotion.py:330-840)
 
 struct MbStats {  // per-device accumulators, all-reduced across ranks by the host (NCCL) when asked
   unsigned long long episodes;
-  unsigned long long steps;
+  unsigned long long steps_reached_sum;  // info["steps_reached"] summed over finished episodes (Stepper, Monkey)
   unsigned long long nonfinite;
   unsigned long long overflow;
   double ret_sum;
   double len_sum;
 };
+
+// one warp per env adds to the per-device statistics; the CPU emulation runs one env at a time
+MB_HD void mb_stat_add(unsigned long long* s, unsigned long long v) {
+#ifdef __CUDACC__
+  atomicAdd(s, v);
+#else
+  *s += v;
+#endif
+}
+MB_HD void mb_stat_add(double* s, double v) {
+#ifdef __CUDACC__
+  atomicAdd(s, v);
+#else
+  *s += v;
+#endif
+}
 
 // warm-start impulses of an env (HBM, MbPhysics::warmstart > 0): zeroed at every reset
 MB_HD void mb_clear_warm(float* warm) {
@@ -88,6 +104,68 @@ MB_HD void mb_clear_warm(float* warm) {
 
 MB_HD int& rec_i(float* rec, int k) { return reinterpret_cast<int*>(rec)[k]; }
 MB_HD int rec_i(const float* rec, int k) { return reinterpret_cast<const int*>(rec)[k]; }
+
+// The end of every env's step(), after the env has written obs, its own record fields and its reward: gym
+// TimeLimit(1000), the episode / diagnostics record, reward / done / truncated, the terminal observation, the episode
+// statistics and the auto-reset (VecEnv convention: on done obs becomes the first observation of the next episode).
+// Per-env differences are compile-time properties of Env: CREDIT_STEPS_REACHED adds `steps_reached` to
+// MbStats::steps_reached_sum at an episode end, and the record's INFO_FIELD (if any) keeps the finished episode's
+// value across the reset.  nonfinite: the state went non-finite (it ended the episode); anybad: non-finite actions.
+template <class Env>
+MB_HD void mb_step_epilogue(typename Env::Mem& S, const MbPhysics& P, float* rec, uint32_t* mt_env, uint32_t* mt_robot,
+                            float* obs, float reward, int env_done, int nonfinite, int steps_reached, int rows,
+                            int ncsum, int overflow, unsigned anybad, float* rew, uint8_t* done, uint8_t* trunc,
+                            float* final_obs, MbStats* stats) {
+  const int elapsed = rec_i(rec, ER_ELAPSED) + 1;
+  int truncated = 0, any_done = env_done;
+  if (elapsed >= 1000) { truncated = !env_done; any_done = 1; }
+  const float epret = rec[ER_EPRET] + reward;
+  const int eplen = rec_i(rec, ER_EPLEN) + 1;
+  MB_LANES(l)
+    if (l == 0) {
+      rec_i(rec, ER_ELAPSED) = elapsed;
+      rec[ER_EPRET] = epret; rec_i(rec, ER_EPLEN) = eplen;
+      rec[ER_ROWS] += (float)rows; rec[ER_CONTACTS] += (float)ncsum; S.step_rows = rows;
+      if (MB_UNLIKELY(overflow > 0)) {  // contacts / rows dropped at MB_MAXC / MB_MAXROW: per env and per device
+        rec_i(rec, ER_OVERFLOW) += overflow;
+        mb_stat_add(&stats->overflow, (unsigned long long)overflow);
+      }
+      *rew = reward; *done = (uint8_t)any_done; *trunc = (uint8_t)truncated;
+    }
+  MB_END
+  if (any_done) {
+    if (final_obs) {
+      MB_LANES(l)
+        for (int i = l; i < Env::OBS; i += 32) final_obs[i] = obs[i];
+      MB_END
+    }
+    MB_LANES(l)
+      if (l == 0) {
+        rec[ER_LAST_EPRET] = epret; rec_i(rec, ER_LAST_EPLEN) = eplen;
+        mb_stat_add(&stats->episodes, 1ull);
+        mb_stat_add(&stats->ret_sum, (double)epret);
+        mb_stat_add(&stats->len_sum, (double)eplen);
+        if constexpr (Env::CREDIT_STEPS_REACHED)
+          mb_stat_add(&stats->steps_reached_sum, (unsigned long long)steps_reached);
+        if (nonfinite) mb_stat_add(&stats->nonfinite, 1ull);
+      }
+    MB_END
+    if constexpr (Env::INFO_FIELD >= 0) {
+      const int keep = rec_i(rec, Env::INFO_FIELD);
+      Env::reset(S, P, rec, mt_env, mt_robot, obs);
+      MB_LANES(l)
+        if (l == 0) rec_i(rec, Env::INFO_FIELD) = keep;  // info of the finished episode stays readable
+      MB_END
+    } else {
+      Env::reset(S, P, rec, mt_env, mt_robot, obs);
+    }
+  }
+  if (anybad) {
+    MB_LANES(l)
+      if (l == 0) mb_stat_add(&stats->nonfinite, 1ull);
+    MB_END
+  }
+}
 
 // ------------------------------------------------------------------------------------------------ MT19937
 // NumPy legacy RandomState stream, warp-cooperative.  mt[0..623] state words, mt[624] position.
@@ -160,12 +238,41 @@ MB_HD void mb_euler(const float* qin, float* rpy) {
 }
 MB_HD float mb_clip5(float x) { return fminf(fmaxf(x, -5.0f), 5.0f); }
 
+// mirrored base pose (robots.py:182-188): joint j of a mirrored robot takes the base angle of joint *src times the
+// returned sign (+-1)
+template <class M> MB_HD float mb_mirror_joint(int j, int mirrored, int* src) {
+  *src = j;
+  float sign = 1.0f;
+  if (mirrored) {
+    for (int k = 0; k < M::NMIRROR; ++k) {
+      if (M::right(k) == j) *src = M::left(k);
+      if (M::left(k) == j) *src = M::right(k);
+    }
+    for (int k = 0; k < M::NNEG; ++k)
+      if (M::neg(k) == j) sign = -1.0f;
+  }
+  return sign;
+}
+
+// WalkerBase.reset pose of joint j (robots.py:182-194): the mirrored base angle plus +-0.1 rad noise from the robot
+// words wr (wr[0..1] drew the mirror coin, joint j's uniform is wr[2 + 2 j]), clipped to +-0.95 normalised
+template <class M> MB_HD float mb_reset_joint(int j, int mirrored, const uint32_t* wr) {
+  int src;
+  const float sign = mb_mirror_joint<M>(j, mirrored, &src);
+  const double ang = sign * M::base_angles(src);
+  const double ds = -0.1 + (0.1 - -0.1) * mt_double(wr + 2 + 2 * j);
+  const double bias = (double)M::lower(j), weight = (double)M::weight(j);
+  double ps = 2 * (ang + ds - bias) / weight - 1;
+  ps = ps > 0.95 ? 0.95 : (ps < -0.95 ? -0.95 : ps);
+  return (float)(weight * (ps + 1) / 2 + bias);
+}
+
 template <class M> struct W3DEnv {
   typedef WarpMem<M> Mem;
   typedef Sim<M> S_;
   typedef M Model;
   enum { NJ = M::NJ, NU = M::NU, OBS = 6 + 2 * M::NJ + M::NFEET + 2, ROBOT_OBS = 6 + 2 * M::NJ + M::NFEET,
-         REC_STRIDE = MB_REC_STRIDE, OBST = 0, ACT = M::NJ, INFO_FIELD = -1 };
+         REC_STRIDE = MB_REC_STRIDE, OBST = 0, ACT = M::NJ, INFO_FIELD = -1, CREDIT_STEPS_REACHED = 0 };
   MB_HD static void load_obstacles(WarpMem<M>&, const float*) {}
 
   // HBM <-> shared
@@ -303,25 +410,7 @@ template <class M> struct W3DEnv {
         rec_i(rec, ER_CLOSE) = 0; rec_i(rec, ER_ELAPSED) = 0; rec[ER_FEET0] = 0.0f; rec[ER_FEET1] = 0.0f;
         rec_i(rec, ER_MIRRORED) = mirrored; rec[ER_EPRET] = 0.0f; rec_i(rec, ER_EPLEN) = 0;
       }
-      if (l < NJ) {
-        // mirrored base pose (robots.py:182-188), +-0.1 rad noise clipped to +-0.95 normalised (robots.py:190-194)
-        int src = l;
-        double sign = 1.0;
-        if (mirrored) {
-          for (int k = 0; k < M::NMIRROR; ++k) {
-            if (M::right(k) == l) src = M::left(k);
-            if (M::left(k) == l) src = M::right(k);
-          }
-          for (int k = 0; k < M::NNEG; ++k)
-            if (M::neg(k) == l) sign = -1.0;
-        }
-        const double ang = sign * (double)M::base_angles(src);
-        const double ds = -0.1 + (0.1 - -0.1) * mt_double(wr + 2 + 2 * l);
-        const double bias = (double)M::lower(l), weight = (double)M::weight(l);
-        double ps = 2 * (ang + ds - bias) / weight - 1;
-        ps = ps > 0.95 ? 0.95 : (ps < -0.95 ? -0.95 : ps);
-        S.q[l] = (float)(weight * (ps + 1) / 2 + bias);
-      }
+      if (l < NJ) S.q[l] = mb_reset_joint<M>(l, mirrored, wr);
       if (l < NU) S.u[l] = 0.0f;
       if (l == 31) {
         S.pos[0] = M::base_x(); S.pos[1] = M::base_y(); S.pos[2] = M::base_z();
@@ -434,61 +523,11 @@ template <class M> struct W3DEnv {
     }
     const float reward = progress + target_bonus - energy + tall - posture - joints_pen;
     target_obs(dist, ang, obs);
-    const int elapsed = rec_i(rec, ER_ELAPSED) + 1;
-    int truncated = 0, any_done = env_done;
-    if (elapsed >= 1000) { truncated = !env_done; any_done = 1; }
-    const float epret = rec[ER_EPRET] + reward;
-    const int eplen = rec_i(rec, ER_EPLEN) + 1;
     MB_LANES(l)
-      if (l == 0) {
-        rec_i(rec, ER_CLOSE) = close; rec[ER_LINPOT] = lp; rec_i(rec, ER_ELAPSED) = elapsed;
-        rec[ER_BODYX] = S.pos[0];
-        rec[ER_EPRET] = epret; rec_i(rec, ER_EPLEN) = eplen;
-        rec[ER_ROWS] += (float)rows; rec[ER_CONTACTS] += (float)ncsum; S.step_rows = rows;
-        if (MB_UNLIKELY(overflow > 0)) {  // contacts / rows dropped at MB_MAXC / MB_MAXROW: per env and per device
-          rec_i(rec, ER_OVERFLOW) += overflow;
-#ifdef __CUDACC__
-          atomicAdd(&stats->overflow, (unsigned long long)overflow);
-#else
-          stats->overflow += overflow;
-#endif
-        }
-        *rew = reward; *done = (uint8_t)any_done; *trunc = (uint8_t)truncated;
-      }
+      if (l == 0) { rec_i(rec, ER_CLOSE) = close; rec[ER_LINPOT] = lp; rec[ER_BODYX] = S.pos[0]; }
     MB_END
-    if (any_done) {
-      if (final_obs) {
-        MB_LANES(l)
-          for (int i = l; i < OBS; i += 32) final_obs[i] = obs[i];
-        MB_END
-      }
-      MB_LANES(l)
-        if (l == 0) {
-          rec[ER_LAST_EPRET] = epret; rec_i(rec, ER_LAST_EPLEN) = eplen;
-#ifdef __CUDACC__
-          atomicAdd(&stats->episodes, 1ull);
-          atomicAdd(&stats->ret_sum, (double)epret);
-          atomicAdd(&stats->len_sum, (double)eplen);
-          if (o.nonfinite) atomicAdd(&stats->nonfinite, 1ull);
-#else
-          stats->episodes += 1; stats->ret_sum += epret; stats->len_sum += eplen;
-          if (o.nonfinite) stats->nonfinite += 1;
-#endif
-        }
-      MB_END
-      reset(S, P, rec, mt_env, mt_robot, obs);
-    }
-    if (anybad) {
-      MB_LANES(l)
-        if (l == 0) {
-#ifdef __CUDACC__
-          atomicAdd(&stats->nonfinite, 1ull);
-#else
-          stats->nonfinite += 1;
-#endif
-        }
-      MB_END
-    }
+    mb_step_epilogue<W3DEnv>(S, P, rec, mt_env, mt_robot, obs, reward, env_done, o.nonfinite, 0, rows, ncsum, overflow,
+                             anybad, rew, done, trunc, final_obs, stats);
     store_state(S, state);
   }
 };
@@ -504,7 +543,7 @@ template <class M, bool PILLAR = false> struct StepperEnv {
   typedef M Model;
   enum { NJ = M::NJ, NU = M::NU, ROBOT_OBS = 6 + 2 * M::NJ + M::NFEET, OBS = ROBOT_OBS + 15, NSTEPS = 20,
          REC_STRIDE = MB_REC_STRIDE_STEPPER, OBST = PILLAR ? MB_OBST_CYLS : MB_OBST_BOXES, ACT = M::NJ,
-         INFO_FIELD = ES_STEPS_REACHED };
+         INFO_FIELD = ES_STEPS_REACHED, CREDIT_STEPS_REACHED = 1 };
   MB_HD static void load_obstacles(Mem& S, const float* rec) { load_boxes(S, rec); }
   MB_HD static void load_state(Mem& S, const float* st) { B_::load_state(S, st); }
   MB_HD static void store_state(const Mem& S, float* st) { B_::store_state(S, st); }
@@ -646,24 +685,7 @@ template <class M, bool PILLAR = false> struct StepperEnv {
         rec_i(rec, ES_NEXT) = 1; rec_i(rec, ES_STEPS_REACHED) = -1;
         rec_i(rec, ES_GAIN_CURRIC) = rec_i(rec, ES_CURRIC);
       }
-      if (l < NJ) {
-        int src = l;
-        double sign = 1.0;
-        if (mirrored) {
-          for (int k = 0; k < M::NMIRROR; ++k) {
-            if (M::right(k) == l) src = M::left(k);
-            if (M::left(k) == l) src = M::right(k);
-          }
-          for (int k = 0; k < M::NNEG; ++k)
-            if (M::neg(k) == l) sign = -1.0;
-        }
-        const double ang = sign * M::base_angles(src);
-        const double ds = -0.1 + (0.1 - -0.1) * mt_double(w + 2 + 2 * l);
-        const double bias = (double)M::lower(l), weight = (double)M::weight(l);
-        double ps = 2 * (ang + ds - bias) / weight - 1;
-        ps = ps > 0.95 ? 0.95 : (ps < -0.95 ? -0.95 : ps);
-        S.q[l] = (float)(weight * (ps + 1) / 2 + bias);
-      }
+      if (l < NJ) S.q[l] = mb_reset_joint<M>(l, mirrored, w);
       if (l < NU) S.u[l] = 0.0f;
       if (l == 31) {
         S.pos[0] = M::stepper_x(); S.pos[1] = M::stepper_y(); S.pos[2] = M::stepper_z();  // robot_init_position, env_locomotion.py:339,845
@@ -807,66 +829,14 @@ template <class M, bool PILLAR = false> struct StepperEnv {
       for (int i = 0; i < 8; ++i) acc += (0.8 + (1.2 - 0.8) * mt_double(w + 2 * i)) * (double)term[i];
       reward = (float)acc;
     }
-    const int elapsed = rec_i(rec, ER_ELAPSED) + 1;
-    int truncated = 0, any_done = env_done;
-    if (elapsed >= 1000) { truncated = !env_done; any_done = 1; }
-    const float epret = rec[ER_EPRET] + reward;
-    const int eplen = rec_i(rec, ER_EPLEN) + 1;
     MB_LANES(l)
       if (l == 0) {
-        rec[ER_LINPOT] = lp; rec_i(rec, ER_ELAPSED) = elapsed;
-        rec[ER_EPRET] = epret; rec_i(rec, ER_EPLEN) = eplen;
-        rec[ER_ROWS] += (float)rows; rec[ER_CONTACTS] += (float)ncsum; S.step_rows = rows;
-        if (MB_UNLIKELY(overflow > 0)) {  // contacts / rows dropped at MB_MAXC / MB_MAXROW: per env and per device
-          rec_i(rec, ER_OVERFLOW) += overflow;
-#ifdef __CUDACC__
-          atomicAdd(&stats->overflow, (unsigned long long)overflow);
-#else
-          stats->overflow += overflow;
-#endif
-        }
+        rec[ER_LINPOT] = lp;
         rec_i(rec, ES_STEPS_REACHED) = (env_done || timestep == 999) ? next : -1;
-        *rew = reward; *done = (uint8_t)any_done; *trunc = (uint8_t)truncated;
       }
     MB_END
-    if (any_done) {
-      if (final_obs) {
-        MB_LANES(l)
-          for (int i = l; i < OBS; i += 32) final_obs[i] = obs[i];
-        MB_END
-      }
-      MB_LANES(l)
-        if (l == 0) {
-          rec[ER_LAST_EPRET] = epret; rec_i(rec, ER_LAST_EPLEN) = eplen;
-#ifdef __CUDACC__
-          atomicAdd(&stats->episodes, 1ull);
-          atomicAdd(&stats->ret_sum, (double)epret);
-          atomicAdd(&stats->len_sum, (double)eplen);
-          atomicAdd(&stats->steps, (unsigned long long)next);
-          if (o.nonfinite) atomicAdd(&stats->nonfinite, 1ull);
-#else
-          stats->episodes += 1; stats->ret_sum += epret; stats->len_sum += eplen; stats->steps += next;
-          if (o.nonfinite) stats->nonfinite += 1;
-#endif
-        }
-      MB_END
-      const int keep = rec_i(rec, ES_STEPS_REACHED);
-      reset(S, P, rec, mt_env, mt_robot, obs);
-      MB_LANES(l)
-        if (l == 0) rec_i(rec, ES_STEPS_REACHED) = keep;  // info of the finished episode stays readable
-      MB_END
-    }
-    if (anybad) {
-      MB_LANES(l)
-        if (l == 0) {
-#ifdef __CUDACC__
-          atomicAdd(&stats->nonfinite, 1ull);
-#else
-          stats->nonfinite += 1;
-#endif
-        }
-      MB_END
-    }
+    mb_step_epilogue<StepperEnv>(S, P, rec, mt_env, mt_robot, obs, reward, env_done, o.nonfinite, next, rows, ncsum,
+                                 overflow, anybad, rew, done, trunc, final_obs, stats);
     B_::store_state(S, state);
   }
 };
@@ -900,7 +870,8 @@ template <class M> struct MonkeyEnv {
   typedef W3DEnv<M> B_;
   typedef M Model;
   enum { NJ = M::NJ, NU = M::NU, ROBOT_OBS = 6 + 2 * M::NJ + M::NFEET, OBS = ROBOT_OBS + 15, NSTEPS = 32, NBARS = 4,
-         REC_STRIDE = MB_REC_STRIDE_MONKEY, OBST = MB_OBST_BARS, ACT = M::NJ, INFO_FIELD = -1 };
+         REC_STRIDE = MB_REC_STRIDE_MONKEY, OBST = MB_OBST_BARS, ACT = M::NJ, INFO_FIELD = -1,
+         CREDIT_STEPS_REACHED = 1 };
   MB_HD static void load_obstacles(Mem& S, const float* rec) { load_bars(S, rec); }
   MB_HD static void load_state(Mem& S, const float* st) { B_::load_state(S, st); }
   MB_HD static void store_state(const Mem& S, float* st) { B_::store_state(S, st); }
@@ -1051,16 +1022,8 @@ template <class M> struct MonkeyEnv {
         rec_i(rec, EM_TIMESTEP) = 0; rec_i(rec, EM_FREEFALL) = 0; rec_i(rec, EM_NEXT) = 2;
       }
       if (l < NJ) {
-        int src = l;
-        float sign = 1.0f;
-        if (mirrored) {
-          for (int k = 0; k < M::NMIRROR; ++k) {
-            if (M::right(k) == l) src = M::left(k);
-            if (M::left(k) == l) src = M::right(k);
-          }
-          for (int k = 0; k < M::NNEG; ++k)
-            if (M::neg(k) == l) sign = -1.0f;
-        }
+        int src;
+        const float sign = mb_mirror_joint<M>(l, mirrored, &src);
         S.q[l] = sign * (float)M::base_angles(src);
       }
       // base_velocity (3, 0, -1) (env_locomotion.py:1154): every lane writes its own coordinate (racecheck: no second
@@ -1183,61 +1146,11 @@ template <class M> struct MonkeyEnv {
     const float reward = progress + step_bonus - fc[swing];
     if (timestep > 180 && next <= 2) env_done = 1;
     tail_obs(S, rec, obs);
-    const int elapsed = rec_i(rec, ER_ELAPSED) + 1;
-    int truncated = 0, any_done = env_done;
-    if (elapsed >= 1000) { truncated = !env_done; any_done = 1; }
-    const float epret = rec[ER_EPRET] + reward;
-    const int eplen = rec_i(rec, ER_EPLEN) + 1;
     MB_LANES(l)
-      if (l == 0) {
-        rec[EM_SWINGPOT] = sp; rec_i(rec, EM_FREEFALL) = freefall; rec_i(rec, ER_ELAPSED) = elapsed;
-        rec[ER_EPRET] = epret; rec_i(rec, ER_EPLEN) = eplen;
-        rec[ER_ROWS] += (float)rows; rec[ER_CONTACTS] += (float)ncsum; S.step_rows = rows;
-        if (MB_UNLIKELY(overflow > 0)) {  // contacts / rows dropped at MB_MAXC / MB_MAXROW: per env and per device
-          rec_i(rec, ER_OVERFLOW) += overflow;
-#ifdef __CUDACC__
-          atomicAdd(&stats->overflow, (unsigned long long)overflow);
-#else
-          stats->overflow += overflow;
-#endif
-        }
-        *rew = reward; *done = (uint8_t)any_done; *trunc = (uint8_t)truncated;
-      }
+      if (l == 0) { rec[EM_SWINGPOT] = sp; rec_i(rec, EM_FREEFALL) = freefall; }
     MB_END
-    if (any_done) {
-      if (final_obs) {
-        MB_LANES(l)
-          for (int i = l; i < OBS; i += 32) final_obs[i] = obs[i];
-        MB_END
-      }
-      MB_LANES(l)
-        if (l == 0) {
-          rec[ER_LAST_EPRET] = epret; rec_i(rec, ER_LAST_EPLEN) = eplen;
-#ifdef __CUDACC__
-          atomicAdd(&stats->episodes, 1ull);
-          atomicAdd(&stats->ret_sum, (double)epret);
-          atomicAdd(&stats->len_sum, (double)eplen);
-          atomicAdd(&stats->steps, (unsigned long long)next);
-          if (o.nonfinite) atomicAdd(&stats->nonfinite, 1ull);
-#else
-          stats->episodes += 1; stats->ret_sum += epret; stats->len_sum += eplen; stats->steps += next;
-          if (o.nonfinite) stats->nonfinite += 1;
-#endif
-        }
-      MB_END
-      reset(S, P, rec, mt_env, mt_robot, obs);
-    }
-    if (anybad) {
-      MB_LANES(l)
-        if (l == 0) {
-#ifdef __CUDACC__
-          atomicAdd(&stats->nonfinite, 1ull);
-#else
-          stats->nonfinite += 1;
-#endif
-        }
-      MB_END
-    }
+    mb_step_epilogue<MonkeyEnv>(S, P, rec, mt_env, mt_robot, obs, reward, env_done, o.nonfinite, next, rows, ncsum,
+                                overflow, anybad, rew, done, trunc, final_obs, stats);
     B_::store_state(S, state);
   }
 };
@@ -1252,7 +1165,8 @@ template <class M> struct CassieEnv {
   typedef W3DEnv<M> B_;
   typedef M Model;
   enum { NJ = M::NJ, NU = M::NU, NO = M::NORDERED, ROBOT_OBS = 6 + 2 * M::NORDERED, OBS = ROBOT_OBS + 2,
-         ACT = M::NPOWERED, REC_STRIDE = MB_REC_STRIDE_CASSIE, OBST = 0, LLC_FRAME_SKIP = 50, INFO_FIELD = -1 };
+         ACT = M::NPOWERED, REC_STRIDE = MB_REC_STRIDE_CASSIE, OBST = 0, LLC_FRAME_SKIP = 50, INFO_FIELD = -1,
+         CREDIT_STEPS_REACHED = 0 };
   MB_HD static void load_obstacles(Mem&, const float*) {}
   MB_HD static void load_state(Mem& S, const float* st) { B_::load_state(S, st); }
   MB_HD static void store_state(const Mem& S, float* st) { B_::store_state(S, st); }
@@ -1415,61 +1329,11 @@ template <class M> struct CassieEnv {
     const float tall = height > 0.6f ? 2.0f : -1.0f;
     if (tall < 0.0f) env_done = 1;
     const float reward = tall + progress;
-    const int elapsed = rec_i(rec, ER_ELAPSED) + 1;
-    int truncated = 0, any_done = env_done;
-    if (elapsed >= 1000) { truncated = !env_done; any_done = 1; }
-    const float epret = rec[ER_EPRET] + reward;
-    const int eplen = rec_i(rec, ER_EPLEN) + 1;
     MB_LANES(l)
-      if (l == 0) {
-        rec[EC_POTENTIAL] = pot; rec[EC_PREVX] = S.pos[0]; rec[EC_PREVY] = S.pos[1];
-        rec_i(rec, ER_ELAPSED) = elapsed;
-        rec[ER_EPRET] = epret; rec_i(rec, ER_EPLEN) = eplen;
-        rec[ER_ROWS] += (float)rows; rec[ER_CONTACTS] += (float)ncsum; S.step_rows = rows;
-        if (MB_UNLIKELY(overflow > 0)) {  // contacts / rows dropped at MB_MAXC / MB_MAXROW: per env and per device
-          rec_i(rec, ER_OVERFLOW) += overflow;
-#ifdef __CUDACC__
-          atomicAdd(&stats->overflow, (unsigned long long)overflow);
-#else
-          stats->overflow += overflow;
-#endif
-        }
-        *rew = reward; *done = (uint8_t)any_done; *trunc = (uint8_t)truncated;
-      }
+      if (l == 0) { rec[EC_POTENTIAL] = pot; rec[EC_PREVX] = S.pos[0]; rec[EC_PREVY] = S.pos[1]; }
     MB_END
-    if (any_done) {
-      if (final_obs) {
-        MB_LANES(l)
-          for (int i = l; i < OBS; i += 32) final_obs[i] = obs[i];
-        MB_END
-      }
-      MB_LANES(l)
-        if (l == 0) {
-          rec[ER_LAST_EPRET] = epret; rec_i(rec, ER_LAST_EPLEN) = eplen;
-#ifdef __CUDACC__
-          atomicAdd(&stats->episodes, 1ull);
-          atomicAdd(&stats->ret_sum, (double)epret);
-          atomicAdd(&stats->len_sum, (double)eplen);
-          if (nonfinite) atomicAdd(&stats->nonfinite, 1ull);
-#else
-          stats->episodes += 1; stats->ret_sum += epret; stats->len_sum += eplen;
-          if (nonfinite) stats->nonfinite += 1;
-#endif
-        }
-      MB_END
-      reset(S, P, rec, mt_env, mt_robot, obs);
-    }
-    if (anybad) {
-      MB_LANES(l)
-        if (l == 0) {
-#ifdef __CUDACC__
-          atomicAdd(&stats->nonfinite, 1ull);
-#else
-          stats->nonfinite += 1;
-#endif
-        }
-      MB_END
-    }
+    mb_step_epilogue<CassieEnv>(S, P, rec, mt_env, mt_robot, obs, reward, env_done, nonfinite, 0, rows, ncsum, overflow,
+                                anybad, rew, done, trunc, final_obs, stats);
     B_::store_state(S, state);
   }
 };

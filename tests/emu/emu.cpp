@@ -12,17 +12,6 @@
 #include "../../mocca_envs_b200/csrc/generated/crab2d_model.h"
 #include "../../mocca_envs_b200/csrc/mb_env.cuh"
 
-typedef W3D_Model WM;
-typedef W3DEnv<WM> WEnv;
-typedef StepperEnv<WM> SEnv;
-typedef WarpMem<WM> WMem;
-typedef MK3D_Model MM;
-typedef MonkeyEnv<MM> MEnv;
-typedef WarpMem<MM> MMem;
-typedef CAS_Model CM;
-typedef CassieEnv<CM> CEnv;
-typedef WarpMem<CM> CMem;
-
 static void default_phys(MbPhysics* p) {
   p->dt = 1.0f / 240.0f; p->substeps = 4; p->iterations = 5; p->gravity = 9.8f; p->erp_contact = 0.9f;
   p->erp_joint = 0.2f; p->linear_slop = 1e-5f; p->lin_damping = 0.04f; p->ang_damping = 0.04f;
@@ -35,177 +24,14 @@ static void default_phys(MbPhysics* p) {
 
 extern "C" {
 int emu_sizeof_phys() { return (int)sizeof(MbPhysics); }
-int emu_sizeof_warpmem() { return (int)sizeof(WMem); }
 void emu_default_phys(MbPhysics* p) { default_phys(p); }
 
-void emu_step_physics(const MbPhysics* p, float* state, const float* tau, int* rows, int* contacts) {
-  static WMem S;
-  memset(&S, 0, sizeof(S));
-  WEnv::load_state(S, state);
-  for (int j = 0; j < WM::NJ; ++j) S.tau[j] = tau[j];
-  int r = 0, nc = 0, ov = 0;
-  Sim<WM>::LaneConst C;
-  Sim<WM>::init_lane_const(C);
-  for (int k = 0; k < p->substeps; ++k) r += Sim<WM>::substep<0>(S, *p, C, &nc, &ov);
-  WEnv::store_state(S, state);
-  *rows = r;
-  *contacts = nc;
-}
-
-// stepSimulation with the warm-start switch: `warm` [MB_NWARM] plays the env's HBM impulse array
-void emu_step_physics_warm(const MbPhysics* p, float* state, const float* tau, float* warm, int* rows, int* contacts) {
-  static WMem S;
-  memset(&S, 0, sizeof(S));
-  S.warm = warm;
-  WEnv::load_state(S, state);
-  for (int j = 0; j < WM::NJ; ++j) S.tau[j] = tau[j];
-  int r = 0, nc = 0, ov = 0;
-  Sim<WM>::LaneConst C;
-  Sim<WM>::init_lane_const(C);
-  for (int k = 0; k < p->substeps; ++k) r += Sim<WM>::substep<0>(S, *p, C, &nc, &ov);
-  WEnv::store_state(S, state);
-  *rows = r;
-  *contacts = nc;
-}
-
-void emu_mass_matrix(const MbPhysics* p, const float* state, float* Mout, float* bias) {
-  static WMem S;
-  memset(&S, 0, sizeof(S));
-  WEnv::load_state(S, state);
-  Sim<WM>::LaneConst C;
-  Sim<WM>::init_lane_const(C);
-  Sim<WM>::kinematics(S, *p, C, true);
-  Sim<WM>::bodies(S, *p);
-  Sim<WM>::mass_matrix_and_rhs(S);
-  const int NU = WM::NU;
-  for (int i = 0; i < NU; ++i) {
-    for (int j = 0; j < NU; ++j) Mout[i * NU + j] = mb_Lget<WM>(S.L, i, j);
-    bias[i] = -S.rhs[i];
-  }
-}
-
-void emu_w3d_reset(const MbPhysics* p, float* state, float* rec, uint32_t* mt_env, uint32_t* mt_robot, float* obs) {
-  static WMem S;
-  memset(&S, 0, sizeof(S));
-  WEnv::reset(S, *p, rec, mt_env, mt_robot, obs);
-  WEnv::store_state(S, state);
-}
-
-void emu_w3d_step(const MbPhysics* p, float* state, float* rec, uint32_t* mt_env, uint32_t* mt_robot,
-                  const float* act, float* obs, float* rew, uint8_t* done, uint8_t* trunc, float* final_obs,
-                  double* stats_out) {
-  static WMem S;
-  memset(&S, 0, sizeof(S));
-  MbStats st;
-  memset(&st, 0, sizeof(st));
-  WEnv::step(S, *p, state, rec, mt_env, mt_robot, act, obs, rew, done, trunc, final_obs, &st);
-  stats_out[0] = (double)st.episodes; stats_out[1] = st.ret_sum; stats_out[2] = st.len_sum;
-  stats_out[3] = (double)st.nonfinite;
-}
-
-// ---- Walker3DStepperEnv
+// ---- Walker3DStepperEnv (also Mike, Pillar)
 void emu_stepper_phys(MbPhysics* p) {
   default_phys(p);
   p->has_ground = 0;
   const float kp = 30000.0f, kd = 1000.0f + 0.1f, denom = p->dt * kp + kd;
   p->box_friction = 1.0f; p->box_erp = p->dt * kp / denom; p->box_cfm = 1.0f / denom;
-}
-int emu_stepper_rec_stride() { return (int)SEnv::REC_STRIDE; }
-
-void emu_stepper_reset(const MbPhysics* p, float* state, float* rec, uint32_t* mt_env, uint32_t* mt_robot, float* obs) {
-  static WMem S;
-  memset(&S, 0, sizeof(S));
-  SEnv::reset(S, *p, rec, mt_env, mt_robot, obs);
-  WEnv::store_state(S, state);
-}
-
-void emu_stepper_step(const MbPhysics* p, float* state, float* rec, uint32_t* mt_env, uint32_t* mt_robot,
-                      const float* act, float* obs, float* rew, uint8_t* done, uint8_t* trunc, float* final_obs,
-                      double* stats_out) {
-  static WMem S;
-  memset(&S, 0, sizeof(S));
-  MbStats st;
-  memset(&st, 0, sizeof(st));
-  SEnv::step(S, *p, state, rec, mt_env, mt_robot, act, obs, rew, done, trunc, final_obs, &st);
-  stats_out[0] = (double)st.episodes; stats_out[1] = st.ret_sum; stats_out[2] = st.len_sum;
-  stats_out[3] = (double)st.nonfinite;
-}
-
-// stepSimulation with the planks described by a Stepper record
-void emu_stepper_step_physics(const MbPhysics* p, float* state, const float* rec, const float* tau, int* rows,
-                              int* contacts) {
-  static WMem S;
-  memset(&S, 0, sizeof(S));
-  WEnv::load_state(S, state);
-  for (int j = 0; j < WM::NJ; ++j) S.tau[j] = tau[j];
-  int r = 0, nc = 0, ov = 0;
-  Sim<WM>::LaneConst C;
-  Sim<WM>::init_lane_const(C);
-  for (int k = 0; k < p->substeps; ++k) {
-    SEnv::load_obstacles(S, rec);
-    r += Sim<WM>::substep<MB_OBST_BOXES>(S, *p, C, &nc, &ov);
-  }
-  WEnv::store_state(S, state);
-  *rows = r;
-  *contacts = nc;
-}
-
-// ---- Monkey3DCustomEnv
-int emu_monkey_rec_stride() { return (int)MEnv::REC_STRIDE; }
-int emu_sizeof_monkey_warpmem() { return (int)sizeof(MMem); }
-
-void emu_monkey_reset(const MbPhysics* p, float* state, float* rec, uint32_t* mt_env, uint32_t* mt_robot, float* obs) {
-  static MMem S;
-  memset(&S, 0, sizeof(S));
-  MEnv::reset(S, *p, rec, mt_env, mt_robot, obs);
-  MEnv::store_state(S, state);
-}
-
-void emu_monkey_step(const MbPhysics* p, float* state, float* rec, uint32_t* mt_env, uint32_t* mt_robot,
-                     const float* act, float* obs, float* rew, uint8_t* done, uint8_t* trunc, float* final_obs,
-                     double* stats_out) {
-  static MMem S;
-  memset(&S, 0, sizeof(S));
-  MbStats st;
-  memset(&st, 0, sizeof(st));
-  MEnv::step(S, *p, state, rec, mt_env, mt_robot, act, obs, rew, done, trunc, final_obs, &st);
-  stats_out[0] = (double)st.episodes; stats_out[1] = st.ret_sum; stats_out[2] = st.len_sum;
-  stats_out[3] = (double)st.nonfinite;
-}
-
-// stepSimulation with the bars described by a Monkey record
-void emu_monkey_step_physics(const MbPhysics* p, float* state, const float* rec, const float* tau, int* rows,
-                             int* contacts) {
-  static MMem S;
-  memset(&S, 0, sizeof(S));
-  MEnv::load_state(S, state);
-  for (int j = 0; j < MM::NJ; ++j) S.tau[j] = tau[j];
-  int r = 0, nc = 0, ov = 0;
-  Sim<MM>::LaneConst C;
-  Sim<MM>::init_lane_const(C);
-  for (int k = 0; k < p->substeps; ++k) {
-    MEnv::load_obstacles(S, rec);
-    r += Sim<MM>::substep<MB_OBST_BARS>(S, *p, C, &nc, &ov);
-  }
-  MEnv::store_state(S, state);
-  *rows = r;
-  *contacts = nc;
-}
-
-void emu_monkey_mass_matrix(const MbPhysics* p, const float* state, float* Mout, float* bias) {
-  static MMem S;
-  memset(&S, 0, sizeof(S));
-  MEnv::load_state(S, state);
-  Sim<MM>::LaneConst C;
-  Sim<MM>::init_lane_const(C);
-  Sim<MM>::kinematics(S, *p, C, true);
-  Sim<MM>::bodies(S, *p);
-  Sim<MM>::mass_matrix_and_rhs(S);
-  const int NU = MM::NU;
-  for (int i = 0; i < NU; ++i) {
-    for (int j = 0; j < NU; ++j) Mout[i * NU + j] = mb_Lget<MM>(S.L, i, j);
-    bias[i] = -S.rhs[i];
-  }
 }
 
 // ---- CassieEnv
@@ -214,132 +40,85 @@ void emu_cassie_phys(MbPhysics* p) {
   p->dt = 0.03f / 50.0f;
   p->substeps = 1;
 }
-int emu_cassie_rec_stride() { return (int)CEnv::REC_STRIDE; }
-int emu_sizeof_cassie_warpmem() { return (int)sizeof(CMem); }
 
-void emu_cassie_reset(const MbPhysics* p, float* state, float* rec, float* obs) {
-  static CMem S;
-  memset(&S, 0, sizeof(S));
-  CEnv::reset(S, *p, rec, nullptr, nullptr, obs);
-  CEnv::store_state(S, state);
-}
-
-void emu_cassie_step(const MbPhysics* p, float* state, float* rec, const float* act, float* obs, float* rew,
-                     uint8_t* done, uint8_t* trunc, float* final_obs, double* stats_out) {
-  static CMem S;
-  memset(&S, 0, sizeof(S));
-  MbStats st;
-  memset(&st, 0, sizeof(st));
-  CEnv::step(S, *p, state, rec, nullptr, nullptr, act, obs, rew, done, trunc, final_obs, &st);
-  stats_out[0] = (double)st.episodes; stats_out[1] = st.ret_sum; stats_out[2] = st.len_sum;
-  stats_out[3] = (double)st.nonfinite;
-}
-
-void emu_cassie_step_physics(const MbPhysics* p, float* state, const float* tau, int* rows, int* contacts) {
-  static CMem S;
-  memset(&S, 0, sizeof(S));
-  CEnv::load_state(S, state);
-  for (int j = 0; j < CM::NJ; ++j) S.tau[j] = tau[j];
-  int r = 0, nc = 0, ov = 0;
-  Sim<CM>::LaneConst C;
-  Sim<CM>::init_lane_const(C);
-  for (int k = 0; k < p->substeps; ++k) r += Sim<CM>::substep<0>(S, *p, C, &nc, &ov);
-  CEnv::store_state(S, state);
-  *rows = r;
-  *contacts = nc;
-}
-
-// the same with the contact points of the last collision pass ([MB_MAXC][MB_POINT_WIDTH], see Sim::substep)
-void emu_cassie_step_physics_points(const MbPhysics* p, float* state, const float* tau, int* rows, int* contacts,
-                                    float* points) {
-  static CMem S;
-  memset(&S, 0, sizeof(S));
-  CEnv::load_state(S, state);
-  for (int j = 0; j < CM::NJ; ++j) S.tau[j] = tau[j];
-  int r = 0, nc = 0, ov = 0;
-  Sim<CM>::LaneConst C;
-  Sim<CM>::init_lane_const(C);
-  for (int k = 0; k < p->substeps; ++k)
-    r += Sim<CM>::substep<0>(S, *p, C, &nc, &ov, k, k == p->substeps - 1 ? points : nullptr);
-  CEnv::store_state(S, state);
-  *rows = r;
-  *contacts = nc;
-}
-
-void emu_cassie_mass_matrix(const MbPhysics* p, const float* state, float* Mout, float* bias) {
-  static CMem S;
-  memset(&S, 0, sizeof(S));
-  CEnv::load_state(S, state);
-  Sim<CM>::LaneConst C;
-  Sim<CM>::init_lane_const(C);
-  Sim<CM>::kinematics(S, *p, C, true);
-  Sim<CM>::bodies(S, *p);
-  Sim<CM>::mass_matrix_and_rhs(S);
-  const int NU = CM::NU;
-  for (int i = 0; i < NU; ++i) {
-    for (int j = 0; j < NU; ++j) Mout[i * NU + j] = mb_Lget<CM>(S.L, i, j);
-    bias[i] = -S.rhs[i];
-  }
-}
-
-// ---- SURVEY 8 f3: more model tables through the same env templates (Child3DCustomEnv-v0, MikeStepperEnv-v0)
-#define EMU_ENV(PFX, MODEL, ENV, OBST)                                                                                \
+// emu_<PFX>_rec_stride / _reset / _step / _step_physics / _mass_matrix of one env kind.
+// step: stats_out[6] = the step's MbStats in the order of mb200_stats (episodes, ret_sum, len_sum, nonfinite,
+// overflow, steps_reached_sum).  step_physics: one stepSimulation with the obstacles of `rec`; `warm` [MB_NWARM] plays
+// the env's HBM warm-start impulses, `points` [MB_MAXC][MB_POINT_WIDTH] receives the contact points of the last
+// collision pass (see Sim::substep); nullptr switches either off.
+#define EMU_ENV(PFX, ENV)                                                                                             \
+  int emu_##PFX##_rec_stride() { return (int)ENV::REC_STRIDE; }                                                       \
   void emu_##PFX##_reset(const MbPhysics* p, float* state, float* rec, uint32_t* mt_env, uint32_t* mt_robot,         \
                          float* obs) {                                                                                \
-    static WarpMem<MODEL> S;                                                                                          \
+    static ENV::Mem S;                                                                                                \
     memset(&S, 0, sizeof(S));                                                                                         \
     ENV::reset(S, *p, rec, mt_env, mt_robot, obs);                                                                    \
-    W3DEnv<MODEL>::store_state(S, state);                                                                             \
+    ENV::store_state(S, state);                                                                                       \
   }                                                                                                                   \
   void emu_##PFX##_step(const MbPhysics* p, float* state, float* rec, uint32_t* mt_env, uint32_t* mt_robot,          \
                         const float* act, float* obs, float* rew, uint8_t* done, uint8_t* trunc, float* final_obs,   \
                         double* stats_out) {                                                                          \
-    static WarpMem<MODEL> S;                                                                                          \
+    static ENV::Mem S;                                                                                                \
     memset(&S, 0, sizeof(S));                                                                                         \
     MbStats st;                                                                                                       \
     memset(&st, 0, sizeof(st));                                                                                       \
     ENV::step(S, *p, state, rec, mt_env, mt_robot, act, obs, rew, done, trunc, final_obs, &st);                       \
     stats_out[0] = (double)st.episodes; stats_out[1] = st.ret_sum; stats_out[2] = st.len_sum;                         \
-    stats_out[3] = (double)st.nonfinite;                                                                              \
+    stats_out[3] = (double)st.nonfinite; stats_out[4] = (double)st.overflow;                                          \
+    stats_out[5] = (double)st.steps_reached_sum;                                                                      \
   }                                                                                                                   \
-  void emu_##PFX##_step_physics(const MbPhysics* p, float* state, const float* rec, const float* tau, int* rows,     \
-                                int* contacts) {                                                                      \
-    static WarpMem<MODEL> S;                                                                                          \
+  void emu_##PFX##_step_physics(const MbPhysics* p, float* state, const float* rec, const float* tau, float* warm,    \
+                                float* points, int* rows, int* contacts) {                                            \
+    typedef Sim<ENV::Model> Sim_;                                                                                     \
+    static ENV::Mem S;                                                                                                \
     memset(&S, 0, sizeof(S));                                                                                         \
-    W3DEnv<MODEL>::load_state(S, state);                                                                              \
-    for (int j = 0; j < MODEL::NJ; ++j) S.tau[j] = tau[j];                                                            \
+    S.warm = warm;                                                                                                    \
+    ENV::load_state(S, state);                                                                                        \
+    for (int j = 0; j < ENV::NJ; ++j) S.tau[j] = tau[j];                                                              \
     int r = 0, nc = 0, ov = 0;                                                                                        \
-    Sim<MODEL>::LaneConst C;                                                                                          \
-    Sim<MODEL>::init_lane_const(C);                                                                                   \
+    Sim_::LaneConst C;                                                                                                \
+    Sim_::init_lane_const(C);                                                                                         \
     for (int k = 0; k < p->substeps; ++k) {                                                                           \
       ENV::load_obstacles(S, rec);                                                                                    \
-      r += Sim<MODEL>::substep<OBST>(S, *p, C, &nc, &ov);                                                             \
+      r += Sim_::substep<ENV::OBST>(S, *p, C, &nc, &ov, k, k == p->substeps - 1 ? points : nullptr);                  \
     }                                                                                                                 \
-    W3DEnv<MODEL>::store_state(S, state);                                                                             \
+    ENV::store_state(S, state);                                                                                       \
     *rows = r;                                                                                                        \
     *contacts = nc;                                                                                                   \
   }                                                                                                                   \
   void emu_##PFX##_mass_matrix(const MbPhysics* p, const float* state, float* Mout, float* bias) {                   \
-    static WarpMem<MODEL> S;                                                                                          \
+    typedef Sim<ENV::Model> Sim_;                                                                                     \
+    static ENV::Mem S;                                                                                                \
     memset(&S, 0, sizeof(S));                                                                                         \
-    W3DEnv<MODEL>::load_state(S, state);                                                                              \
-    Sim<MODEL>::LaneConst C;                                                                                          \
-    Sim<MODEL>::init_lane_const(C);                                                                                   \
-    Sim<MODEL>::kinematics(S, *p, C, true);                                                                           \
-    Sim<MODEL>::bodies(S, *p);                                                                                        \
-    Sim<MODEL>::mass_matrix_and_rhs(S);                                                                               \
-    const int NU = MODEL::NU;                                                                                         \
+    ENV::load_state(S, state);                                                                                        \
+    Sim_::LaneConst C;                                                                                                \
+    Sim_::init_lane_const(C);                                                                                         \
+    Sim_::kinematics(S, *p, C, true);                                                                                 \
+    Sim_::bodies(S, *p);                                                                                              \
+    Sim_::mass_matrix_and_rhs(S);                                                                                     \
+    const int NU = ENV::NU;                                                                                           \
     for (int i = 0; i < NU; ++i) {                                                                                    \
-      for (int j = 0; j < NU; ++j) Mout[i * NU + j] = mb_Lget<MODEL>(S.L, i, j);                                      \
+      for (int j = 0; j < NU; ++j) Mout[i * NU + j] = mb_Lget<ENV::Model>(S.L, i, j);                                 \
       bias[i] = -S.rhs[i];                                                                                            \
     }                                                                                                                 \
   }
-EMU_ENV(child, CH3D_Model, W3DEnv<CH3D_Model>, 0)
-EMU_ENV(mike, MIKE_Model, StepperEnv<MIKE_Model>, MB_OBST_BOXES)
-// the planar walkers (Walker2DCustomEnv-v0, Crab2DCustomEnv-v0)
-EMU_ENV(walker2d, W2D_Model, W3DEnv<W2D_Model>, 0)
-EMU_ENV(crab2d, CR2D_Model, W3DEnv<CR2D_Model>, 0)
-// plank_class = "Pillar": the PILLAR instantiation of the stepper template
-typedef StepperEnv<WM, true> SEnvPillar;
-EMU_ENV(pillar, WM, SEnvPillar, MB_OBST_CYLS)
+
+typedef W3DEnv<W3D_Model> W3DKind;
+typedef StepperEnv<W3D_Model> StepperKind;
+typedef StepperEnv<W3D_Model, true> PillarKind;  // plank_class = "Pillar"
+typedef MonkeyEnv<MK3D_Model> MonkeyKind;
+typedef CassieEnv<CAS_Model> CassieKind;
+typedef W3DEnv<CH3D_Model> ChildKind;  // Child3DCustomEnv-v0
+typedef StepperEnv<MIKE_Model> MikeKind;  // MikeStepperEnv-v0
+typedef W3DEnv<W2D_Model> Walker2DKind;
+typedef W3DEnv<CR2D_Model> Crab2DKind;
+EMU_ENV(w3d, W3DKind)
+EMU_ENV(stepper, StepperKind)
+EMU_ENV(pillar, PillarKind)
+EMU_ENV(monkey, MonkeyKind)
+EMU_ENV(cassie, CassieKind)
+EMU_ENV(child, ChildKind)
+EMU_ENV(mike, MikeKind)
+EMU_ENV(walker2d, Walker2DKind)
+EMU_ENV(crab2d, Crab2DKind)
 }

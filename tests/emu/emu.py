@@ -39,63 +39,50 @@ def lib():
     return _lib
 
 
-def default_phys():
+def _phys(fn):
     p = Phys()
-    lib().emu_default_phys(C.byref(p))
+    getattr(lib(), fn)(C.byref(p))
     return p
 
 
+def default_phys():
+    return _phys("emu_default_phys")
+
+
+def cassie_phys():
+    return _phys("emu_cassie_phys")
+
+
 def _fp(a):
-    return a.ctypes.data_as(C.c_void_p)
+    return None if a is None else a.ctypes.data_as(C.c_void_p)
 
 
-def step_physics(p, state, tau):
-    state = np.ascontiguousarray(state, dtype=np.float32).copy()
-    buf = np.zeros(64, dtype=np.float32)
-    buf[: len(state)] = state
-    tau = np.ascontiguousarray(tau, dtype=np.float32)
-    rows, nc = C.c_int(0), C.c_int(0)
-    lib().emu_step_physics(C.byref(p), _fp(buf), _fp(tau), C.byref(rows), C.byref(nc))
-    return buf[: len(state)].copy(), rows.value, nc.value
+class EmuEnv:
+    """One env through the emulated kernel source: emu_<prefix>_* in emu.cpp (record layout: ER_* and the kind's
+    additions in mb_env.cuh).  A subclass per env kind names its prefix, dimensions and physics defaults."""
 
+    prefix = None
+    obs_dim = act_dim = n_dof = None
+    phys_fn = "emu_default_phys"  # the kind's physics defaults (as mb200_create sets them)
+    aliased = 1  # ER_ALIASED: the robot draws from the env stream until the env is re-seeded
 
-def step_physics_warm(p, state, tau, warm):
-    """stepSimulation with MbPhysics.warmstart: `warm` (float32[384], updated in place) carries the contact impulses."""
-    state = np.ascontiguousarray(state, dtype=np.float32).copy()
-    buf = np.zeros(64, dtype=np.float32)
-    buf[: len(state)] = state
-    tau = np.ascontiguousarray(tau, dtype=np.float32)
-    rows, nc = C.c_int(0), C.c_int(0)
-    lib().emu_step_physics_warm(C.byref(p), _fp(buf), _fp(tau), _fp(warm), C.byref(rows), C.byref(nc))
-    return buf[: len(state)].copy(), rows.value, nc.value
-
-
-def mass_matrix(p, state, nu):
-    buf = np.zeros(64, dtype=np.float32)
-    buf[: len(state)] = state
-    M = np.zeros((nu, nu), dtype=np.float32)
-    b = np.zeros(nu, dtype=np.float32)
-    lib().emu_mass_matrix(C.byref(p), _fp(buf), _fp(M), _fp(b))
-    return M, b
-
-
-class EmuW3D:
-    prefix = "w3d"  # emu_<prefix>_reset / _step in emu.cpp
-
-    def __init__(self, mt_state, obs_dim=52, act_dim=21, phys=None):
-        self.p = phys or default_phys()
+    def __init__(self, mt_state=None, phys=None):
+        self.p = phys or _phys(self.phys_fn)
         self.state = np.zeros(64, dtype=np.float32)
-        self.rec = np.zeros(32, dtype=np.float32)
+        self.rec = np.zeros(self._call("rec_stride"), dtype=np.float32)
+        self.rec.view(np.int32)[11] = self.aliased
         self.mt = np.zeros((2, 640), dtype=np.uint32)
-        self.mt[0, :625] = mt_state
+        if mt_state is not None:
+            self.mt[0, :625] = mt_state
         self.mt[1, 624] = 624
-        self.rec.view(np.int32)[11] = 1  # ER_ALIASED
-        self.obs_dim, self.act_dim = obs_dim, act_dim
-        self.stats = np.zeros(4)
+        self.stats = np.zeros(6)  # accumulated MbStats, in the order of mb200_stats
+
+    def _call(self, what, *args):
+        return getattr(lib(), "emu_%s_%s" % (self.prefix, what))(*args)
 
     def reset(self):
         obs = np.zeros(self.obs_dim, dtype=np.float32)
-        getattr(lib(), "emu_%s_reset" % self.prefix)(C.byref(self.p), _fp(self.state), _fp(self.rec), _fp(self.mt[0]), _fp(self.mt[1]), _fp(obs))
+        self._call("reset", C.byref(self.p), _fp(self.state), _fp(self.rec), _fp(self.mt[0]), _fp(self.mt[1]), _fp(obs))
         return obs
 
     def step(self, act):
@@ -105,12 +92,35 @@ class EmuW3D:
         rew = np.zeros(1, dtype=np.float32)
         done = np.zeros(1, dtype=np.uint8)
         trunc = np.zeros(1, dtype=np.uint8)
-        st = np.zeros(4)
-        getattr(lib(), "emu_%s_step" % self.prefix)(C.byref(self.p), _fp(self.state), _fp(self.rec), _fp(self.mt[0]),
-                                                    _fp(self.mt[1]), _fp(act), _fp(obs), _fp(rew), _fp(done), _fp(trunc),
-                                                    _fp(fin), _fp(st))
+        st = np.zeros(6)
+        self._call("step", C.byref(self.p), _fp(self.state), _fp(self.rec), _fp(self.mt[0]), _fp(self.mt[1]),
+                   _fp(act), _fp(obs), _fp(rew), _fp(done), _fp(trunc), _fp(fin), _fp(st))
         self.stats += st
         return obs, float(rew[0]), bool(done[0]), bool(trunc[0]), fin
+
+    def step_physics(self, tau, warm=None, points=None):
+        """One stepSimulation of self.state (in place) with the obstacles of self.rec, joint torques `tau` held.
+        `warm` (float32[384], updated in place) switches warm starting on; `points` (float32[16, 10]) receives the
+        contact points of the last collision pass.  Returns (rows, contacts)."""
+        tau = np.ascontiguousarray(tau, dtype=np.float32)
+        rows, nc = C.c_int(0), C.c_int(0)
+        self._call("step_physics", C.byref(self.p), _fp(self.state), _fp(self.rec), _fp(tau), _fp(warm), _fp(points),
+                   C.byref(rows), C.byref(nc))
+        return rows.value, nc.value
+
+    def mass_matrix(self):
+        """(mass matrix, bias forces) at self.state."""
+        nu = 6 + self.n_dof
+        M = np.zeros((nu, nu), dtype=np.float32)
+        b = np.zeros(nu, dtype=np.float32)
+        self._call("mass_matrix", C.byref(self.p), _fp(self.state), _fp(M), _fp(b))
+        return M, b
+
+
+class EmuW3D(EmuEnv):
+    """Walker3DCustomEnv."""
+    prefix = "w3d"
+    obs_dim, act_dim, n_dof = 52, 21, 21
 
 
 class EmuChild(EmuW3D):
@@ -121,91 +131,36 @@ class EmuChild(EmuW3D):
 class EmuWalker2D(EmuW3D):
     """Walker2DCustomEnv-v0: the Walker3DCustomEnv template on the planar walker2d table."""
     prefix = "walker2d"
-
-    def __init__(self, mt_state, phys=None):
-        super().__init__(mt_state, obs_dim=24, act_dim=7, phys=phys)
+    obs_dim, act_dim, n_dof = 24, 7, 7
 
 
 class EmuCrab2D(EmuW3D):
     """Crab2DCustomEnv-v0."""
     prefix = "crab2d"
-
-    def __init__(self, mt_state, phys=None):
-        super().__init__(mt_state, obs_dim=22, act_dim=6, phys=phys)
+    obs_dim, act_dim, n_dof = 22, 6, 6
 
 
-def model_step_physics(prefix, p, state, tau, rec=None):
-    """stepSimulation through emu_<prefix>_step_physics (child: ground plane; mike: the planks of a Stepper record)."""
-    buf = np.zeros(64, dtype=np.float32)
-    buf[: len(state)] = state
-    tau = np.ascontiguousarray(tau, dtype=np.float32)
-    rec = np.zeros(192, dtype=np.float32) if rec is None else rec
-    rows, nc = C.c_int(0), C.c_int(0)
-    getattr(lib(), "emu_%s_step_physics" % prefix)(C.byref(p), _fp(buf), _fp(rec), _fp(tau), C.byref(rows), C.byref(nc))
-    return buf[: len(state)].copy(), rows.value, nc.value
-
-
-def model_mass_matrix(prefix, p, state, nu=27):
-    buf = np.zeros(64, dtype=np.float32)
-    buf[: len(state)] = state
-    M = np.zeros((nu, nu), dtype=np.float32)
-    b = np.zeros(nu, dtype=np.float32)
-    getattr(lib(), "emu_%s_mass_matrix" % prefix)(C.byref(p), _fp(buf), _fp(M), _fp(b))
-    return M, b
-
-
-def stepper_phys():
-    p = Phys()
-    lib().emu_stepper_phys(C.byref(p))
-    return p
-
-
-class EmuStepper:
-    """Walker3DStepperEnv through the emulated kernel source (record layout: ER_* / ES_* in mb_env.cuh)."""
+class EmuStepper(EmuEnv):
+    """Walker3DStepperEnv (record additions ES_*)."""
 
     prefix = "stepper"
+    obs_dim, act_dim, n_dof = 65, 21, 21
+    phys_fn = "emu_stepper_phys"
 
     ES_NEXT, ES_COUNT, ES_STOP, ES_SETSTOP, ES_TIMESTEP, ES_CURRIC, ES_PLANKIDX, ES_STEPS = 22, 23, 24, 25, 26, 27, 28, 31
     ES_BOX, ES_TERRAIN = 32, 68
 
-    def __init__(self, mt_state, curriculum=0):
-        self.p = stepper_phys()
-        self.state = np.zeros(64, dtype=np.float32)
-        self.stride = lib().emu_stepper_rec_stride()
-        self.rec = np.zeros(self.stride, dtype=np.float32)
-        self.mt = np.zeros((2, 640), dtype=np.uint32)
-        self.mt[0, :625] = mt_state
-        self.mt[1, 624] = 624
-        self.rec.view(np.int32)[11] = 1  # ER_ALIASED
+    def __init__(self, mt_state=None, curriculum=0, phys=None):
+        super().__init__(mt_state, phys)
         self.rec.view(np.int32)[self.ES_CURRIC] = curriculum
-        self.obs_dim = 65
-
-    def reset(self):
-        obs = np.zeros(self.obs_dim, dtype=np.float32)
-        getattr(lib(), "emu_%s_reset" % self.prefix)(C.byref(self.p), _fp(self.state), _fp(self.rec), _fp(self.mt[0]), _fp(self.mt[1]), _fp(obs))
-        return obs
-
-    def step(self, act):
-        act = np.ascontiguousarray(act, dtype=np.float32)
-        obs = np.zeros(self.obs_dim, dtype=np.float32)
-        fin = np.zeros(self.obs_dim, dtype=np.float32)
-        rew = np.zeros(1, dtype=np.float32)
-        done = np.zeros(1, dtype=np.uint8)
-        trunc = np.zeros(1, dtype=np.uint8)
-        st = np.zeros(4)
-        getattr(lib(), "emu_%s_step" % self.prefix)(C.byref(self.p), _fp(self.state), _fp(self.rec), _fp(self.mt[0]),
-                                                    _fp(self.mt[1]), _fp(act), _fp(obs), _fp(rew), _fp(done), _fp(trunc),
-                                                    _fp(fin), _fp(st))
-        return obs, float(rew[0]), bool(done[0]), bool(trunc[0]), fin
 
     def terrain(self):
         return self.rec[self.ES_TERRAIN:self.ES_TERRAIN + 120].reshape(20, 6)
 
-    def step_physics(self, tau):
-        tau = np.ascontiguousarray(tau, dtype=np.float32)
-        rows, nc = C.c_int(0), C.c_int(0)
-        getattr(lib(), "emu_%s_step_physics" % self.prefix)(C.byref(self.p), _fp(self.state), _fp(self.rec), _fp(tau), C.byref(rows), C.byref(nc))
-        return rows.value, nc.value
+
+class EmuPillar(EmuStepper):
+    """Walker3DStepperEnv with plank_class = "Pillar"."""
+    prefix = "pillar"
 
 
 class EmuMike(EmuStepper):
@@ -213,116 +168,25 @@ class EmuMike(EmuStepper):
     prefix = "mike"
 
 
-class EmuMonkey:
-    """Monkey3DCustomEnv through the emulated kernel source (record layout: ER_* / EM_* in mb_env.cuh)."""
+class EmuMonkey(EmuEnv):
+    """Monkey3DCustomEnv (record additions EM_*)."""
+
+    prefix = "monkey"
+    obs_dim, act_dim, n_dof = 69, 23, 23
 
     EM_NEXT, EM_FREEFALL, EM_TIMESTEP, EM_SWING, EM_PIVOT, EM_SWINGPOT, EM_BARIDX, EM_BAR, EM_TERRAIN = \
         22, 23, 24, 25, 26, 27, 28, 32, 64
 
-    def __init__(self, mt_state):
-        self.p = default_phys()
-        self.state = np.zeros(64, dtype=np.float32)
-        self.stride = lib().emu_monkey_rec_stride()
-        self.rec = np.zeros(self.stride, dtype=np.float32)
-        self.mt = np.zeros((2, 640), dtype=np.uint32)
-        self.mt[0, :625] = mt_state
-        self.mt[1, 624] = 624
-        self.rec.view(np.int32)[11] = 1  # ER_ALIASED
-        self.obs_dim, self.act_dim = 69, 23
-
-    def reset(self):
-        obs = np.zeros(self.obs_dim, dtype=np.float32)
-        lib().emu_monkey_reset(C.byref(self.p), _fp(self.state), _fp(self.rec), _fp(self.mt[0]), _fp(self.mt[1]), _fp(obs))
-        return obs
-
-    def step(self, act):
-        act = np.ascontiguousarray(act, dtype=np.float32)
-        obs = np.zeros(self.obs_dim, dtype=np.float32)
-        fin = np.zeros(self.obs_dim, dtype=np.float32)
-        rew = np.zeros(1, dtype=np.float32)
-        done = np.zeros(1, dtype=np.uint8)
-        trunc = np.zeros(1, dtype=np.uint8)
-        st = np.zeros(4)
-        lib().emu_monkey_step(C.byref(self.p), _fp(self.state), _fp(self.rec), _fp(self.mt[0]), _fp(self.mt[1]),
-                              _fp(act), _fp(obs), _fp(rew), _fp(done), _fp(trunc), _fp(fin), _fp(st))
-        return obs, float(rew[0]), bool(done[0]), bool(trunc[0]), fin
-
     def terrain(self):
         return self.rec[self.EM_TERRAIN:self.EM_TERRAIN + 128].reshape(32, 4)
 
-    def step_physics(self, tau):
-        tau = np.ascontiguousarray(tau, dtype=np.float32)
-        rows, nc = C.c_int(0), C.c_int(0)
-        lib().emu_monkey_step_physics(C.byref(self.p), _fp(self.state), _fp(self.rec), _fp(tau), C.byref(rows), C.byref(nc))
-        return rows.value, nc.value
 
+class EmuCassie(EmuEnv):
+    """CassieEnv-v0 (record additions EC_*).  Deterministic: its MT streams are never drawn from."""
 
-def monkey_mass_matrix(p, state, nu=29):
-    buf = np.zeros(64, dtype=np.float32)
-    buf[: len(state)] = state
-    M = np.zeros((nu, nu), dtype=np.float32)
-    b = np.zeros(nu, dtype=np.float32)
-    lib().emu_monkey_mass_matrix(C.byref(p), _fp(buf), _fp(M), _fp(b))
-    return M, b
-
-
-def cassie_phys():
-    p = Phys()
-    lib().emu_cassie_phys(C.byref(p))
-    return p
-
-
-class EmuCassie:
-    """CassieEnv-v0 through the emulated kernel source (record layout: ER_* / EC_* in mb_env.cuh)."""
+    prefix = "cassie"
+    obs_dim, act_dim, n_dof = 36, 10, 18
+    phys_fn = "emu_cassie_phys"
+    aliased = 0
 
     EC_POTENTIAL, EC_JVEL = 22, 32
-
-    def __init__(self):
-        self.p = cassie_phys()
-        self.state = np.zeros(64, dtype=np.float32)
-        self.stride = lib().emu_cassie_rec_stride()
-        self.rec = np.zeros(self.stride, dtype=np.float32)
-        self.obs_dim, self.act_dim, self.n_dof = 36, 10, 18
-
-    def reset(self):
-        obs = np.zeros(self.obs_dim, dtype=np.float32)
-        lib().emu_cassie_reset(C.byref(self.p), _fp(self.state), _fp(self.rec), _fp(obs))
-        return obs
-
-    def step(self, act):
-        act = np.ascontiguousarray(act, dtype=np.float32)
-        obs = np.zeros(self.obs_dim, dtype=np.float32)
-        fin = np.zeros(self.obs_dim, dtype=np.float32)
-        rew = np.zeros(1, dtype=np.float32)
-        done = np.zeros(1, dtype=np.uint8)
-        trunc = np.zeros(1, dtype=np.uint8)
-        st = np.zeros(4)
-        lib().emu_cassie_step(C.byref(self.p), _fp(self.state), _fp(self.rec), _fp(act), _fp(obs), _fp(rew), _fp(done),
-                              _fp(trunc), _fp(fin), _fp(st))
-        return obs, float(rew[0]), bool(done[0]), bool(trunc[0]), fin
-
-    def step_physics(self, tau):
-        tau = np.ascontiguousarray(tau, dtype=np.float32)
-        rows, nc = C.c_int(0), C.c_int(0)
-        lib().emu_cassie_step_physics(C.byref(self.p), _fp(self.state), _fp(tau), C.byref(rows), C.byref(nc))
-        return rows.value, nc.value
-
-
-def cassie_step_physics_points(p, state, tau):
-    """(state after, rows, contacts, points[16, 10]) of one Cassie stepSimulation through the kernel source."""
-    buf = np.zeros(64, dtype=np.float32)
-    buf[: len(state)] = state
-    tau = np.ascontiguousarray(tau, dtype=np.float32)
-    rows, nc = C.c_int(0), C.c_int(0)
-    pts = np.zeros((16, 10), dtype=np.float32)
-    lib().emu_cassie_step_physics_points(C.byref(p), _fp(buf), _fp(tau), C.byref(rows), C.byref(nc), _fp(pts))
-    return buf[: len(state)].copy(), rows.value, nc.value, pts
-
-
-def cassie_mass_matrix(p, state, nu=24):
-    buf = np.zeros(64, dtype=np.float32)
-    buf[: len(state)] = state
-    M = np.zeros((nu, nu), dtype=np.float32)
-    b = np.zeros(nu, dtype=np.float32)
-    lib().emu_cassie_mass_matrix(C.byref(p), _fp(buf), _fp(M), _fp(b))
-    return M, b

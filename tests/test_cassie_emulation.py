@@ -64,12 +64,13 @@ def test_cassie_mass_matrix_and_bias(cassie_table, oracle_mod):
     A = t["n_dof"]
     m = O.model_from_table(t)
     p = O.cassie_params()
-    ep = E.cassie_phys()
+    emu = E.EmuCassie()
     rng = np.random.RandomState(0)
     for row in random_states(_rand_table(t), rng, 6):
         s = oracle_state(O, A, row)
         M = O.mass_matrix(m, s)
-        Me, be = E.cassie_mass_matrix(ep, row.astype(np.float32), 6 + A)
+        emu.state[:len(row)] = row
+        Me, be = emu.mass_matrix()
         assert np.abs(Me - M).max() / np.abs(M).max() < 1e-6
         acc = O.forward_dynamics(m, p, s, np.zeros(A), with_damping=True)
         bias = -M @ acc
@@ -137,7 +138,7 @@ def test_cassie_hull_self_collision(cassie_table, oracle_mod):
     p = O.cassie_params()
     p_off = O.cassie_params()
     p_off.self_collision = 0
-    pe = E.cassie_phys()
+    emu = E.EmuCassie()
     rng = np.random.RandomState(3)
     states = cassie_hull_contact_states(O, t, rng, 24)
     errs, effect = [], []
@@ -145,7 +146,10 @@ def test_cassie_hull_self_collision(cassie_table, oracle_mod):
         s = oracle_state(O, A, st.astype(np.float64))
         c0 = O.collide(m, p, s)
         c, rows_ref = O.step_physics(m, p, s, np.zeros(A))
-        out, rows, nc, pts = E.cassie_step_physics_points(pe, st, np.zeros(A, dtype=np.float32))
+        emu.state[:len(st)] = st
+        pts = np.zeros((16, 10), dtype=np.float32)
+        rows, nc = emu.step_physics(np.zeros(A, dtype=np.float32), points=pts)
+        out = emu.state[:len(st)].copy()
         assert nc == c.n and rows == rows_ref
         for k in range(c0.n):
             if c0.partner[k] >= 1000:

@@ -19,12 +19,13 @@ def test_mass_matrix_and_bias(name, child_table, mike_table, oracle_mod):
     A = t["n_dof"]
     m = O.model_from_table(t)
     p = O.default_params()
-    ep = E.default_phys()
+    emu = {"child": E.EmuChild, "mike": E.EmuMike}[name](phys=E.default_phys())
     rng = np.random.RandomState(0)
     for row in random_states(t, rng, 4):
         s = oracle_state(O, A, row)
         M = O.mass_matrix(m, s)
-        Me, be = E.model_mass_matrix(name, ep, row.astype(np.float32), 6 + A)
+        emu.state[:len(row)] = row
+        Me, be = emu.mass_matrix()
         assert np.abs(Me - M).max() / np.abs(M).max() < 1e-6
         acc = O.forward_dynamics(m, p, s, np.zeros(A), with_damping=True)
         bias = -M @ acc
@@ -51,7 +52,7 @@ def test_child_contact_step(child_table, oracle_mod):
     A = t["n_dof"]
     m = O.model_from_table(t)
     p = O.default_params()
-    ep = E.default_phys()
+    emu = E.EmuChild()
     rng = np.random.RandomState(2)
     gain = np.array(t["gain"])
     worst, with_contacts = 0.0, 0
@@ -64,11 +65,12 @@ def test_child_contact_step(child_table, oracle_mod):
         tau = 0.3 * gain * rng.uniform(-1, 1, A)
         s = oracle_state(O, A, row)
         c, rows = O.step_physics(m, p, s, tau)
-        out, erows, enc = E.model_step_physics("child", ep, row.astype(np.float32), tau)
+        emu.state[:len(row)] = row
+        erows, enc = emu.step_physics(tau)
         assert enc == c.n
         assert abs(rows - erows) <= 2
         with_contacts += c.n > 0
-        worst = max(worst, state_error(out, O.state_vector(s, A)))
+        worst = max(worst, state_error(emu.state[:len(row)], O.state_vector(s, A)))
     assert with_contacts >= 6
     assert worst < 2e-3, worst
 

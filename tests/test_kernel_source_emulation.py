@@ -15,12 +15,13 @@ def test_mass_matrix_and_bias(walker_table, oracle_mod):
     A = t["n_dof"]
     m = O.model_from_table(t)
     p = O.default_params()
-    ep = E.default_phys()
+    emu = E.EmuW3D()
     rng = np.random.RandomState(0)
     for row in random_states(t, rng, 6):
         s = oracle_state(O, A, row)
         M = O.mass_matrix(m, s)
-        Me, be = E.mass_matrix(ep, row.astype(np.float32), 6 + A)
+        emu.state[:len(row)] = row
+        Me, be = emu.mass_matrix()
         assert np.abs(Me - M).max() / np.abs(M).max() < 1e-6
         acc = O.forward_dynamics(m, p, s, np.zeros(A), with_damping=True)
         bias = -M @ acc
@@ -33,16 +34,17 @@ def test_contact_free_step(walker_table, oracle_mod):
     A = t["n_dof"]
     m = O.model_from_table(t)
     p = O.default_params()
-    ep = E.default_phys()
+    emu = E.EmuW3D()
     rng = np.random.RandomState(1)
     gain = np.array(t["gain"])
     for row in random_states(t, rng, 8, spin=0.5, margin=0.35):
         tau = gain * rng.uniform(-1, 1, A)
         s = oracle_state(O, A, row)
         _, rows = O.step_physics(m, p, s, tau)
-        out, erows, _ = E.step_physics(ep, row.astype(np.float32), tau)
+        emu.state[:len(row)] = row
+        erows, _ = emu.step_physics(tau)
         assert rows == erows == 0
-        assert state_error(out, O.state_vector(s, A)) < 1e-4
+        assert state_error(emu.state[:len(row)], O.state_vector(s, A)) < 1e-4
 
 
 def test_contact_step(walker_table, oracle_mod):
@@ -51,7 +53,7 @@ def test_contact_step(walker_table, oracle_mod):
     A = t["n_dof"]
     m = O.model_from_table(t)
     p = O.default_params()
-    ep = E.default_phys()
+    emu = E.EmuW3D()
     rng = np.random.RandomState(2)
     gain = np.array(t["gain"])
     worst = 0.0
@@ -60,10 +62,11 @@ def test_contact_step(walker_table, oracle_mod):
         tau = 0.3 * gain * rng.uniform(-1, 1, A)
         s = oracle_state(O, A, row)
         c, rows = O.step_physics(m, p, s, tau)
-        out, erows, enc = E.step_physics(ep, row.astype(np.float32), tau)
+        emu.state[:len(row)] = row
+        erows, enc = emu.step_physics(tau)
         assert enc == c.n
         assert abs(rows - erows) <= 2  # a limit row can flip at an exact boundary
-        worst = max(worst, state_error(out, O.state_vector(s, A)))
+        worst = max(worst, state_error(emu.state[:len(row)], O.state_vector(s, A)))
     assert worst < 2e-3, worst
 
 
@@ -75,9 +78,10 @@ def test_self_contact_step(walker_table, oracle_mod):
     A = t["n_dof"]
     m = O.model_from_table(t)
     p = O.default_params()
-    ep = E.default_phys()
+    emu = E.EmuW3D()
     off = E.default_phys()
     off.self_collision = 0
+    emu_off = E.EmuW3D(phys=off)
     rng = np.random.RandomState(3)
     gain = np.array(t["gain"])
     worst, worst_off = 0.0, 0.0
@@ -85,12 +89,14 @@ def test_self_contact_step(walker_table, oracle_mod):
         tau = gain * rng.uniform(-1, 1, A)
         s = oracle_state(O, A, row)
         c, rows = O.step_physics(m, p, s, tau)
-        out, erows, enc = E.step_physics(ep, row.astype(np.float32), tau)
+        emu.state[:len(row)] = row
+        erows, enc = emu.step_physics(tau)
         assert enc == c.n
         assert abs(rows - erows) <= 2
-        worst = max(worst, state_error(out, O.state_vector(s, A)))
-        out2, _, _ = E.step_physics(off, row.astype(np.float32), tau)
-        worst_off = max(worst_off, state_error(out2, O.state_vector(s, A)))
+        worst = max(worst, state_error(emu.state[:len(row)], O.state_vector(s, A)))
+        emu_off.state[:len(row)] = row
+        emu_off.step_physics(tau)
+        worst_off = max(worst_off, state_error(emu_off.state[:len(row)], O.state_vector(s, A)))
     assert worst < 2e-3, worst
     assert worst_off > 0.1, worst_off
 
@@ -231,12 +237,8 @@ def test_stepper_pillar_class(walker_table, oracle_mod):
     from tests.helpers import oracle_state, state_error
 
     O, t = oracle_mod, walker_table
-
-    class EmuPillar(E.EmuStepper):
-        prefix = "pillar"
-
     outs = {}
-    for cls, emu_cls in (("LargePlank", E.EmuStepper), ("Pillar", EmuPillar)):
+    for cls, emu_cls in (("LargePlank", E.EmuStepper), ("Pillar", E.EmuPillar)):
         env = O.Walker3DStepperOracle(t, seed=2, curriculum=0, plank_class=cls)
         emu = emu_cls(_mt_row(O, 2), curriculum=0)
         env.reset()
@@ -290,10 +292,12 @@ def test_warm_start_switch(walker_table, oracle_mod):
             s = oracle_state(O, A, st.astype(np.float64))
             warm_o = (C.c_double * 384)()
             warm_e = np.zeros(384, dtype=np.float32)
-            se = st.copy()
+            emu = E.EmuW3D(phys=pe)
+            emu.state[:len(st)] = st
             for k in range(3):
                 O.step_physics(m, p, s, tau.astype(np.float64), warm=warm_o)
-                se, _, _ = (E.step_physics_warm(pe, se, tau, warm_e) if f > 0 else E.step_physics(pe, se, tau))
+                emu.step_physics(tau, warm=warm_e if f > 0 else None)
+            se = emu.state[:len(st)].copy()
             outs[f] = (O.state_vector(s, A), se)
             if f > 0:
                 worst_on = max(worst_on, state_error(se, O.state_vector(s, A)))

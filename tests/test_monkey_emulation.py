@@ -17,12 +17,13 @@ def test_monkey_mass_matrix_and_bias(monkey_table, oracle_mod):
     A = t["n_dof"]
     m = O.model_from_table(t)
     p = O.default_params()
-    ep = E.default_phys()
+    emu = E.EmuMonkey()
     rng = np.random.RandomState(0)
     for row in random_states(t, rng, 6):
         s = oracle_state(O, A, row)
         M = O.mass_matrix(m, s)
-        Me, be = E.monkey_mass_matrix(ep, row.astype(np.float32), 6 + A)
+        emu.state[:len(row)] = row
+        Me, be = emu.mass_matrix()
         assert np.abs(Me - M).max() / np.abs(M).max() < 1e-6
         acc = O.forward_dynamics(m, p, s, np.zeros(A), with_damping=True)
         bias = -M @ acc

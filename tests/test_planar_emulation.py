@@ -55,12 +55,13 @@ def test_tables(walker2d_table, crab2d_table):
 def test_mass_matrix_and_bias(name, walker2d_table, crab2d_table, oracle_mod):
     O, t = oracle_mod, _table(name, walker2d_table, crab2d_table)
     A = t["n_dof"]
-    m, p, ep = O.model_from_table(t), O.default_params(), E.default_phys()
+    m, p, emu = O.model_from_table(t), O.default_params(), {"walker2d": E.EmuWalker2D, "crab2d": E.EmuCrab2D}[name]()
     rng = np.random.RandomState(0)
     for row in _planar_states(t, rng, 4):
         s = oracle_state(O, A, row)
         M = O.mass_matrix(m, s)
-        Me, be = E.model_mass_matrix(name, ep, row.astype(np.float32), 6 + A)
+        emu.state[:len(row)] = row
+        Me, be = emu.mass_matrix()
         assert np.abs(Me - M).max() / np.abs(M).max() < 1e-6
         # the in-plane block {omega_y, v_x, v_z, joints} decouples exactly from {omega_x, omega_z, v_y}
         inp, outp = [1, 3, 5] + list(range(6, 6 + A)), [0, 2, 4]

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Bit-level fingerprint of the kernel source (g++ lane-loop emulation, tests/emu): seeded rollouts of every env kind,
-CRC of every observation / reward / state.  A refactoring that only moves addressing around (no change of the
+CRC of every observation / reward / state / record and of the accumulated episode statistics.  A refactoring that only moves addressing around (no change of the
 floating-point operations or their order) must leave every line unchanged:
 
     python tools/emu_hash.py > /tmp/before.txt;  <edit>;  python tools/emu_hash.py | diff /tmp/before.txt -
@@ -25,7 +25,8 @@ def rollout(env, act_dim, steps, seed, scale=1.0):
     ndone = 0
     for _ in range(steps):
         obs, rew, done, trunc, fin = env.step(scale * rng.uniform(-1, 1, act_dim))
-        crc = zlib.crc32(obs.tobytes() + np.float32(rew).tobytes() + env.state.tobytes(), crc)
+        crc = zlib.crc32(obs.tobytes() + np.float32(rew).tobytes() + env.state.tobytes() + env.rec.tobytes() +
+                         env.stats.tobytes(), crc)
         ndone += done
     return "%08x episodes %d" % (crc, ndone)
 
@@ -41,6 +42,7 @@ def main():
         print("crab2d", seed, rollout(emu.EmuCrab2D(m), 6, steps, seed))
         for cur in (0, 9):
             print("stepper c%d" % cur, seed, rollout(emu.EmuStepper(m, cur), 21, steps, seed, 0.4))
+        print("pillar", seed, rollout(emu.EmuPillar(m, 5), 21, steps, seed, 0.4))
         print("mike", seed, rollout(emu.EmuMike(m, 5), 21, steps, seed, 0.4))
         print("monkey", seed, rollout(emu.EmuMonkey(m), 23, steps, seed))
         print("cassie", seed, rollout(emu.EmuCassie(), 10, max(steps // 6, 4), seed))
