@@ -44,8 +44,7 @@ class Physics(C.Structure):
 
 def _units():
     """(source, object, dependencies) of every translation unit."""
-    units = [(os.path.join(CSRC, "mb200.cu"), os.path.join(BUILD_DIR, "mb200.o"),
-              COMMON + [os.path.join(CSRC, "generated", "walker3d_model.h")])]
+    units = [(os.path.join(CSRC, "mb200.cu"), os.path.join(BUILD_DIR, "mb200.o"), COMMON)]
     for kind, model in KINDS.items():
         units.append((os.path.join(CSRC, "kinds", kind + ".cu"), os.path.join(BUILD_DIR, kind + ".o"),
                       COMMON + [os.path.join(CSRC, "generated", model + "_model.h")]))

@@ -11,7 +11,6 @@
 #include <string>
 
 #include "../../include/mocca_b200.h"
-#include "generated/walker3d_model.h" /* only for sizing asserts; the kernels live in kinds/ */
 #include "mb_kind.cuh"
 
 static thread_local std::string g_err;
@@ -22,33 +21,26 @@ static int fail(const std::string& m) { g_err = m; return -1; }
     if (e_ != cudaSuccess) return fail(std::string(#x) + ": " + cudaGetErrorString(e_));                 \
   } while (0)
 
-// KIND_CHILD / KIND_MIKE (SURVEY 8 f3) run the Walker3DCustomEnv / Walker3DStepperEnv templates on other model tables
-// KIND_WALKER2D / KIND_CRAB2D: the planar walkers (free base that stays in the x-z plane) on the Walker3DCustomEnv template
-enum { KIND_CUSTOM = 0, KIND_STEPPER = 1, KIND_MONKEY = 2, KIND_CASSIE = 3, KIND_CHILD = 4, KIND_MIKE = 5,
-       KIND_WALKER2D = 6, KIND_CRAB2D = 7, KIND_COUNT };
-static bool custom_family(int kind) {
-  return kind == KIND_CUSTOM || kind == KIND_CHILD || kind == KIND_WALKER2D || kind == KIND_CRAB2D;
-}
-static bool stepper_family(int kind) { return kind == KIND_STEPPER || kind == KIND_MIKE; }
-
+// Every kernel table (csrc/kinds/*.cu).  An env id runs its "" variant; plank_class = Pillar switches a stepper
+// batch to its "pillar" variant (the cylinder-stone instantiation).
 extern const MbKindOps mb_kind_walker3d_custom, mb_kind_walker3d_stepper, mb_kind_walker3d_stepper_pillar,
     mb_kind_monkey3d_custom, mb_kind_cassie, mb_kind_child3d_custom, mb_kind_walker2d_custom, mb_kind_crab2d_custom,
     mb_kind_mike_stepper, mb_kind_mike_stepper_pillar;
-// [kind][pillar]
-static const MbKindOps* const g_kinds[KIND_COUNT][2] = {
-    {&mb_kind_walker3d_custom, nullptr},
-    {&mb_kind_walker3d_stepper, &mb_kind_walker3d_stepper_pillar},
-    {&mb_kind_monkey3d_custom, nullptr},
-    {&mb_kind_cassie, nullptr},
-    {&mb_kind_child3d_custom, nullptr},
-    {&mb_kind_mike_stepper, &mb_kind_mike_stepper_pillar},
-    {&mb_kind_walker2d_custom, nullptr},
-    {&mb_kind_crab2d_custom, nullptr},
+static const MbKindOps* const g_kinds[] = {
+    &mb_kind_walker3d_custom, &mb_kind_walker3d_stepper, &mb_kind_walker3d_stepper_pillar, &mb_kind_monkey3d_custom,
+    &mb_kind_cassie,          &mb_kind_child3d_custom,   &mb_kind_mike_stepper,            &mb_kind_mike_stepper_pillar,
+    &mb_kind_walker2d_custom, &mb_kind_crab2d_custom,
 };
 
+static const MbKindOps* find_kind(const char* env_id, const char* variant) {
+  if (env_id)
+    for (const MbKindOps* k : g_kinds)
+      if (strcmp(k->env_id, env_id) == 0 && strcmp(k->variant, variant) == 0) return k;
+  return nullptr;
+}
+
 struct mb200_env {
-  int kind;        // KIND_*
-  bool pillar;     // stepper family: plank_class = Pillar, launch the cylinder-stone instantiation
+  const MbKindOps* ops;  // the kernels this batch launches
   int warps;       // envs per CTA of this kind's kernels
   int rec_stride;  // floats per env in `rec`
   int n, device;
@@ -89,7 +81,6 @@ struct mb200_env {
   long long launches;
   size_t smem;
 };
-static const MbKindOps* ops_of(const mb200_env* e) { return g_kinds[e->kind][e->pillar ? 1 : 0]; }
 
 // ------------------------------------------------------------------------------------------------ kernels
 // Second half of the counting sort (the histogram was filled by the step kernel): every CTA scans the 256 bins into
@@ -148,67 +139,75 @@ extern "C" {
 
 const char* mb200_last_error(void) { return g_err.c_str(); }
 
-void mb200_default_physics(mb200_physics* p) {
-  p->dt = 1.0f / 240.0f;
-  p->substeps = 4;
-  p->iterations = 5;
-  p->gravity = 9.8f;
-  p->erp_contact = 0.9f;
-  p->erp_joint = 0.2f;
-  p->linear_slop = 1e-5f;
-  p->lin_damping = 0.04f;
-  p->ang_damping = 0.04f;
-  p->max_coord_vel = 100.0f;
-  p->limit_max_impulse = 100.0f;
-  p->split_threshold = -0.04f;
-  p->residual_threshold = 1e-7f;
-  p->ground_friction = 0.8f;
-  p->has_ground = 1;
-  p->self_collision = 1;
-  p->warmstart = 0.0f;
-}
+void mb200_default_physics(mb200_physics* p) { mb_default_physics(p); }
 
 void mb200_default_physics_for(const char* env_id, mb200_physics* p) {
-  mb200_default_physics(p);
-  if (env_id && strcmp(env_id, "CassieEnv-v0") == 0) {
-    // control_step 0.03 / llc_frame_skip 50 / sim_frame_skip 1 (env_cassie.py:287-289, env_base.py:81); one
-    // stepSimulation = one substep, 50 of them per env step
-    p->dt = 0.03f / 50.0f;
-    p->substeps = 1;
-  }
-}
-
-static void to_internal(const mb200_physics& p, MbPhysics* q) {
-  q->dt = p.dt; q->substeps = p.substeps; q->iterations = p.iterations; q->gravity = p.gravity;
-  q->erp_contact = p.erp_contact; q->erp_joint = p.erp_joint; q->linear_slop = p.linear_slop;
-  q->lin_damping = p.lin_damping; q->ang_damping = p.ang_damping; q->max_coord_vel = p.max_coord_vel;
-  q->limit_max_impulse = p.limit_max_impulse; q->split_threshold = p.split_threshold;
-  q->residual_threshold = p.residual_threshold; q->ground_friction = p.ground_friction; q->has_ground = p.has_ground;
-  q->box_friction = 1.0f; q->box_erp = p.erp_contact; q->box_cfm = 0.0f; q->bar_friction = 0.5f;
-  q->self_collision = p.self_collision;
-  q->warmstart = p.warmstart > 0.0f ? p.warmstart : 0.0f;
+  mb_default_physics(p);
+  if (const MbKindOps* K = find_kind(env_id, "")) K->default_physics(*p);
 }
 
 static int grid_for(const mb200_env* e) { return (e->n + e->warps - 1) / e->warps; }
+
+// the device arrays of a new handle, all zeroed (info: -1 = not reported) except the identity launch order
+static int alloc_buffers(mb200_env* e) {
+  const size_t n = (size_t)e->n_pad;
+  CUDA_OK(cudaMalloc(&e->dummy_obs, (size_t)2 * MB_WARPS_MAX * e->obs_dim * sizeof(float)));
+  CUDA_OK(cudaMalloc(&e->dummy_rew, MB_WARPS_MAX * sizeof(float)));
+  CUDA_OK(cudaMalloc(&e->dummy_flag, 2 * MB_WARPS_MAX));
+  CUDA_OK(cudaMalloc(&e->dummy_stats, sizeof(MbStats)));
+  CUDA_OK(cudaMemset(e->dummy_stats, 0, sizeof(MbStats)));
+  CUDA_OK(cudaMalloc(&e->state, n * MB_STATE_STRIDE * sizeof(float)));
+  CUDA_OK(cudaMalloc(&e->rec, n * e->rec_stride * sizeof(float)));
+  CUDA_OK(cudaMalloc(&e->mt, n * 2 * MB_MT_STRIDE * sizeof(uint32_t)));
+  CUDA_OK(cudaMalloc(&e->stats, sizeof(MbStats)));
+  CUDA_OK(cudaMalloc(&e->order, n * sizeof(int)));
+  CUDA_OK(cudaMalloc(&e->key, n * sizeof(int)));
+  CUDA_OK(cudaMalloc(&e->hist, 2 * 256 * sizeof(int)));
+  CUDA_OK(cudaMalloc(&e->cursor, 2 * 256 * sizeof(int)));
+  CUDA_OK(cudaMemset(e->key, 0, n * sizeof(int)));
+  CUDA_OK(cudaMemset(e->hist, 0, 2 * 256 * sizeof(int)));
+  CUDA_OK(cudaMemset(e->cursor, 0, 2 * 256 * sizeof(int)));
+  {
+    int* ident = (int*)malloc(n * sizeof(int));
+    if (!ident) return fail("mb200_create: host allocation failed");
+    for (size_t i = 0; i < n; ++i) ident[i] = (int)i;
+    cudaError_t ce = cudaMemcpy(e->order, ident, n * sizeof(int), cudaMemcpyHostToDevice);
+    free(ident);
+    CUDA_OK(ce);
+  }
+  CUDA_OK(cudaMalloc(&e->stage_act, n * e->act_dim * sizeof(float)));
+  CUDA_OK(cudaMalloc(&e->stage_obs, n * e->obs_dim * sizeof(float)));
+  CUDA_OK(cudaMalloc(&e->stage_rew, n * sizeof(float)));
+  CUDA_OK(cudaMalloc(&e->stage_done, n));
+  CUDA_OK(cudaMalloc(&e->stage_trunc, n));
+  CUDA_OK(cudaEventCreateWithFlags(&e->host_done, cudaEventDisableTiming));
+  CUDA_OK(cudaMemset(e->state, 0, n * MB_STATE_STRIDE * sizeof(float)));
+  CUDA_OK(cudaMemset(e->rec, 0, n * e->rec_stride * sizeof(float)));
+  CUDA_OK(cudaMemset(e->mt, 0, n * 2 * MB_MT_STRIDE * sizeof(uint32_t)));
+  CUDA_OK(cudaMemset(e->stats, 0, sizeof(MbStats)));
+  CUDA_OK(cudaMalloc(&e->stage_mask, n));
+  if (e->phys.warmstart > 0.0f) {
+    CUDA_OK(cudaMalloc(&e->warm, n * MB_NWARM * sizeof(float)));
+    CUDA_OK(cudaMemset(e->warm, 0, n * MB_NWARM * sizeof(float)));
+  }
+  CUDA_OK(cudaMalloc(&e->info, n * sizeof(int)));
+  CUDA_OK(cudaMemset(e->info, 0xff, n * sizeof(int)));
+  return 0;
+}
 
 void mb200_destroy(mb200_env* e);
 
 int mb200_create(const char* env_id, int n_envs, int device, const mb200_physics* physics, mb200_env** out) {
   if (!out) return fail("mb200_create: out is NULL");
   *out = nullptr;
-  int kind = -1;
-  if (env_id && strcmp(env_id, "Walker3DCustomEnv-v0") == 0) kind = KIND_CUSTOM;
-  if (env_id && strcmp(env_id, "Walker3DStepperEnv-v0") == 0) kind = KIND_STEPPER;
-  if (env_id && strcmp(env_id, "Monkey3DCustomEnv-v0") == 0) kind = KIND_MONKEY;
-  if (env_id && strcmp(env_id, "CassieEnv-v0") == 0) kind = KIND_CASSIE;
-  if (env_id && strcmp(env_id, "Child3DCustomEnv-v0") == 0) kind = KIND_CHILD;
-  if (env_id && strcmp(env_id, "Walker2DCustomEnv-v0") == 0) kind = KIND_WALKER2D;
-  if (env_id && strcmp(env_id, "Crab2DCustomEnv-v0") == 0) kind = KIND_CRAB2D;
-  if (env_id && strcmp(env_id, "MikeStepperEnv-v0") == 0) kind = KIND_MIKE;
-  if (kind < 0)
-    return fail(std::string("mb200_create: unsupported env id '") + (env_id ? env_id : "(null)") +
-                "' (built: Walker3DCustomEnv-v0, Walker3DStepperEnv-v0, Monkey3DCustomEnv-v0, CassieEnv-v0, "
-                "Child3DCustomEnv-v0, MikeStepperEnv-v0, Walker2DCustomEnv-v0, Crab2DCustomEnv-v0)");
+  const MbKindOps* K = find_kind(env_id, "");
+  if (!K) {
+    std::string built;
+    for (const MbKindOps* k : g_kinds)
+      if (!*k->variant) built += (built.empty() ? "" : ", ") + std::string(k->env_id);
+    return fail(std::string("mb200_create: unsupported env id '") + (env_id ? env_id : "(null)") + "' (built: " +
+                built + ")");
+  }
   if (n_envs <= 0) return fail("mb200_create: n_envs must be positive");
   int count = 0;
   CUDA_OK(cudaGetDeviceCount(&count));
@@ -219,13 +218,18 @@ int mb200_create(const char* env_id, int n_envs, int device, const mb200_physics
     return fail("mb200_create: device is not compute capability 10.x; this library carries sm_100a code only and has "
                 "no CPU or other-arch fallback");
   CUDA_OK(cudaSetDevice(device));
+  // opt every kernel of the env id (each variant) in to the dynamic shared memory of a full-width CTA (the attribute
+  // is per kernel, not per handle, and several env kinds can live in one process)
+  for (const MbKindOps* k : g_kinds)
+    if (strcmp(k->env_id, env_id) == 0) {
+      const cudaError_t pe = k->prepare();
+      if (pe != cudaSuccess) return fail(std::string("mb200_create: shared-memory opt-in: ") + cudaGetErrorString(pe));
+    }
   mb200_env* e = new mb200_env();
   memset(e, 0, sizeof(*e));
   e->n = n_envs;
   e->device = device;
-  e->kind = kind;
-  e->pillar = false;
-  const MbKindOps* K = g_kinds[kind][0];
+  e->ops = K;
   const int nj = K->nj;
   e->rec_stride = K->rec_stride; e->obs_dim = K->obs_dim; e->act_dim = K->act_dim;
   e->warps = K->warps;
@@ -247,82 +251,16 @@ int mb200_create(const char* env_id, int n_envs, int device, const mb200_physics
   mb200_physics p;
   mb200_default_physics_for(env_id, &p);
   if (physics) p = *physics;
-  to_internal(p, &e->phys);
-  if (stepper_family(kind)) {
-    // remove_ground=True (env_locomotion.py:359); planks: lateralFriction 1.0, contactStiffness 30000,
-    // contactDamping 1000 (bullet_objects.py:64-72) -> per-contact erp / cfm (SURVEY App. B.4); Bullet sums both
-    // bodies' contact damping and a link's default is 0.1
-    e->phys.has_ground = 0;
-    const float kp = 30000.0f, kd = 1000.0f + 0.1f, denom = e->phys.dt * kp + kd;
-    e->phys.box_friction = 1.0f;
-    e->phys.box_erp = e->phys.dt * kp / denom;
-    e->phys.box_cfm = 1.0f / denom;
-  }
+  mb_to_internal(p, &e->phys);
+  K->fix_physics(e->phys);
   e->smem = K->smem_per_env * e->warps;
-  // opt every kernel of the kind in to the dynamic shared memory of a full-width CTA (the attribute is per kernel, not
-  // per handle, and several env kinds can live in one process)
-  for (int v = 0; v < 2; ++v)
-    if (g_kinds[kind][v]) {
-      const cudaError_t pe = g_kinds[kind][v]->prepare();
-      if (pe != cudaSuccess) { delete e; return fail(std::string("mb200_create: shared-memory opt-in: ") + cudaGetErrorString(pe)); }
-    }
   e->n_pad = grid_for(e) * e->warps;
-  const size_t n = (size_t)e->n_pad;
-#undef CUDA_OK
-#define CUDA_OK(x)                                                                                       \
-  do {                                                                                                   \
-    cudaError_t e_ = (x);                                                                                \
-    if (e_ != cudaSuccess) { mb200_destroy(e); return fail(std::string(#x) + ": " + cudaGetErrorString(e_)); } \
-  } while (0)
-  CUDA_OK(cudaMalloc(&e->dummy_obs, (size_t)2 * MB_WARPS_MAX * e->obs_dim * sizeof(float)));
-  CUDA_OK(cudaMalloc(&e->dummy_rew, MB_WARPS_MAX * sizeof(float)));
-  CUDA_OK(cudaMalloc(&e->dummy_flag, 2 * MB_WARPS_MAX));
-  CUDA_OK(cudaMalloc(&e->dummy_stats, sizeof(MbStats)));
-  CUDA_OK(cudaMemset(e->dummy_stats, 0, sizeof(MbStats)));
-  CUDA_OK(cudaMalloc(&e->state, n * MB_STATE_STRIDE * sizeof(float)));
-  CUDA_OK(cudaMalloc(&e->rec, n * e->rec_stride * sizeof(float)));
-  CUDA_OK(cudaMalloc(&e->mt, n * 2 * MB_MT_STRIDE * sizeof(uint32_t)));
-  CUDA_OK(cudaMalloc(&e->stats, sizeof(MbStats)));
-  CUDA_OK(cudaMalloc(&e->order, n * sizeof(int)));
-  CUDA_OK(cudaMalloc(&e->key, n * sizeof(int)));
-  CUDA_OK(cudaMalloc(&e->hist, 2 * 256 * sizeof(int)));
-  CUDA_OK(cudaMalloc(&e->cursor, 2 * 256 * sizeof(int)));
-  CUDA_OK(cudaMemset(e->key, 0, n * sizeof(int)));
-  CUDA_OK(cudaMemset(e->hist, 0, 2 * 256 * sizeof(int)));
-  CUDA_OK(cudaMemset(e->cursor, 0, 2 * 256 * sizeof(int)));
-  {
-    int* ident = (int*)malloc(n * sizeof(int));
-    if (!ident) { mb200_destroy(e); return fail("mb200_create: host allocation failed"); }
-    for (size_t i = 0; i < n; ++i) ident[i] = (int)i;
-    cudaError_t ce = cudaMemcpy(e->order, ident, n * sizeof(int), cudaMemcpyHostToDevice);
-    free(ident);
-    CUDA_OK(ce);
-  }
   e->sort_every = 1;
   if (const char* sv = getenv("MB200_SORT_EVERY")) e->sort_every = atoi(sv);
-  CUDA_OK(cudaMalloc(&e->stage_act, n * e->act_dim * sizeof(float)));
-  CUDA_OK(cudaMalloc(&e->stage_obs, n * e->obs_dim * sizeof(float)));
-  CUDA_OK(cudaMalloc(&e->stage_rew, n * sizeof(float)));
-  CUDA_OK(cudaMalloc(&e->stage_done, n));
-  CUDA_OK(cudaMalloc(&e->stage_trunc, n));
-  CUDA_OK(cudaEventCreateWithFlags(&e->host_done, cudaEventDisableTiming));
-  CUDA_OK(cudaMemset(e->state, 0, n * MB_STATE_STRIDE * sizeof(float)));
-  CUDA_OK(cudaMemset(e->rec, 0, n * e->rec_stride * sizeof(float)));
-  CUDA_OK(cudaMemset(e->mt, 0, n * 2 * MB_MT_STRIDE * sizeof(uint32_t)));
-  CUDA_OK(cudaMemset(e->stats, 0, sizeof(MbStats)));
-  CUDA_OK(cudaMalloc(&e->stage_mask, n));
-  if (e->phys.warmstart > 0.0f) {
-    CUDA_OK(cudaMalloc(&e->warm, n * MB_NWARM * sizeof(float)));
-    CUDA_OK(cudaMemset(e->warm, 0, n * MB_NWARM * sizeof(float)));
+  if (alloc_buffers(e)) {
+    mb200_destroy(e);
+    return -1;
   }
-  CUDA_OK(cudaMalloc(&e->info, n * sizeof(int)));
-  CUDA_OK(cudaMemset(e->info, 0xff, n * sizeof(int)));
-#undef CUDA_OK
-#define CUDA_OK(x)                                                                                       \
-  do {                                                                                                   \
-    cudaError_t e_ = (x);                                                                                \
-    if (e_ != cudaSuccess) return fail(std::string(#x) + ": " + cudaGetErrorString(e_));                 \
-  } while (0)
   *out = e;
   return 0;
 }
@@ -354,41 +292,31 @@ int mb200_seed(mb200_env* e, const uint32_t* mt_host, int at_construction) {
   CUDA_OK(cudaSetDevice(e->device));
   CUDA_OK(cudaDeviceSynchronize());
   const size_t n = (size_t)e->n_pad, nreal = (size_t)e->n;
-  if (!at_construction) {
-    // EnvBase.seed rebinds only the env's RandomState: an aliased robot keeps drawing from the OLD stream,
-    // which therefore moves to the robot slot (quirk Q1)
-    uint32_t* tmp = (uint32_t*)malloc(n * 2 * MB_MT_STRIDE * sizeof(uint32_t));
-    float* rec = (float*)malloc(n * e->rec_stride * sizeof(float));
-    if (!tmp || !rec) { free(tmp); free(rec); return fail("mb200_seed: host allocation failed"); }
+  uint32_t* tmp = (uint32_t*)calloc(n * 2 * MB_MT_STRIDE, sizeof(uint32_t));
+  float* rec = (float*)malloc(n * e->rec_stride * sizeof(float));
+  if (!tmp || !rec) { free(tmp); free(rec); return fail("mb200_seed: host allocation failed"); }
+  if (!at_construction)
     CUDA_OK(cudaMemcpy(tmp, e->mt, n * 2 * MB_MT_STRIDE * sizeof(uint32_t), cudaMemcpyDeviceToHost));
-    CUDA_OK(cudaMemcpy(rec, e->rec, n * e->rec_stride * sizeof(float), cudaMemcpyDeviceToHost));
-    for (size_t i = 0; i < n; ++i) {
-      int* ri = reinterpret_cast<int*>(rec + i * e->rec_stride);
-      if (ri[ER_ALIASED]) {
-        memcpy(tmp + (i * 2 + 1) * MB_MT_STRIDE, tmp + (i * 2) * MB_MT_STRIDE, 625 * sizeof(uint32_t));
-        ri[ER_ALIASED] = 0;
-      }
-      memcpy(tmp + (i * 2) * MB_MT_STRIDE, mt_host + (i % nreal) * 625, 625 * sizeof(uint32_t));
+  CUDA_OK(cudaMemcpy(rec, e->rec, n * e->rec_stride * sizeof(float), cudaMemcpyDeviceToHost));
+  for (size_t i = 0; i < n; ++i) {
+    int& aliased = reinterpret_cast<int*>(rec + i * e->rec_stride)[ER_ALIASED];
+    uint32_t* env_mt = tmp + (i * 2) * MB_MT_STRIDE;
+    uint32_t* robot_mt = env_mt + MB_MT_STRIDE;
+    if (at_construction) {
+      robot_mt[624] = 624;  // the robot draws from the env's stream (env_base.py:93)
+      aliased = 1;
+    } else if (aliased) {
+      // EnvBase.seed rebinds only the env's RandomState: an aliased robot keeps drawing from the OLD stream,
+      // which therefore moves to the robot slot (quirk Q1)
+      memcpy(robot_mt, env_mt, 625 * sizeof(uint32_t));
+      aliased = 0;
     }
-    CUDA_OK(cudaMemcpy(e->mt, tmp, n * 2 * MB_MT_STRIDE * sizeof(uint32_t), cudaMemcpyHostToDevice));
-    CUDA_OK(cudaMemcpy(e->rec, rec, n * e->rec_stride * sizeof(float), cudaMemcpyHostToDevice));
-    free(tmp);
-    free(rec);
-  } else {
-    uint32_t* tmp = (uint32_t*)calloc(n * 2 * MB_MT_STRIDE, sizeof(uint32_t));
-    float* rec = (float*)malloc(n * e->rec_stride * sizeof(float));
-    if (!tmp || !rec) { free(tmp); free(rec); return fail("mb200_seed: host allocation failed"); }
-    CUDA_OK(cudaMemcpy(rec, e->rec, n * e->rec_stride * sizeof(float), cudaMemcpyDeviceToHost));
-    for (size_t i = 0; i < n; ++i) {
-      memcpy(tmp + (i * 2) * MB_MT_STRIDE, mt_host + (i % nreal) * 625, 625 * sizeof(uint32_t));
-      tmp[(i * 2 + 1) * MB_MT_STRIDE + 624] = 624;
-      reinterpret_cast<int*>(rec + i * e->rec_stride)[ER_ALIASED] = 1;
-    }
-    CUDA_OK(cudaMemcpy(e->mt, tmp, n * 2 * MB_MT_STRIDE * sizeof(uint32_t), cudaMemcpyHostToDevice));
-    CUDA_OK(cudaMemcpy(e->rec, rec, n * e->rec_stride * sizeof(float), cudaMemcpyHostToDevice));
-    free(tmp);
-    free(rec);
+    memcpy(env_mt, mt_host + (i % nreal) * 625, 625 * sizeof(uint32_t));
   }
+  CUDA_OK(cudaMemcpy(e->mt, tmp, n * 2 * MB_MT_STRIDE * sizeof(uint32_t), cudaMemcpyHostToDevice));
+  CUDA_OK(cudaMemcpy(e->rec, rec, n * e->rec_stride * sizeof(float), cudaMemcpyHostToDevice));
+  free(tmp);
+  free(rec);
   return 0;
 }
 
@@ -396,7 +324,7 @@ int mb200_reset(mb200_env* e, const uint8_t* mask_dev, float* obs_dev, void* str
   if (!e || !obs_dev) return fail("mb200_reset: NULL argument");
   CUDA_OK(cudaSetDevice(e->device));
   const LaunchDims d = {grid_for(e), e->warps * 32, e->smem, (cudaStream_t)stream};
-  ops_of(e)->reset(d, e->n, e->phys, e->state, e->rec, e->mt, mask_dev, obs_dev, e->dummy_obs, e->warm);
+  e->ops->reset(d, e->n, e->phys, e->state, e->rec, e->mt, mask_dev, obs_dev, e->dummy_obs, e->warm);
   e->launches++;
   CUDA_OK(cudaGetLastError());
   return 0;
@@ -481,7 +409,7 @@ static int step_impl(mb200_env* e, const float* act_dev, float* obs_dev, float* 
   a.info = e->info;
   a.warm = e->warm;
   const LaunchDims d = {grid_for(e), e->warps * 32, e->smem, (cudaStream_t)stream};
-  ops_of(e)->step(a, host != nullptr, d);
+  e->ops->step(a, host != nullptr, d);
   e->launches++;
   e->steps++;
   CUDA_OK(cudaGetLastError());
@@ -621,7 +549,7 @@ static int step_physics_impl(mb200_env* e, const float* tau_dev, int* rows_dev, 
   if (!e || !tau_dev) return fail("mb200_step_physics: NULL argument");
   CUDA_OK(cudaSetDevice(e->device));
   const LaunchDims d = {grid_for(e), e->warps * 32, e->smem, (cudaStream_t)stream};
-  ops_of(e)->physics(d, e->n, e->phys, e->state, e->rec, tau_dev, rows_dev, contacts_dev, points_dev, e->warm);
+  e->ops->physics(d, e->n, e->phys, e->state, e->rec, tau_dev, rows_dev, contacts_dev, points_dev, e->warm);
   e->launches++;
   CUDA_OK(cudaGetLastError());
   return 0;
@@ -644,7 +572,7 @@ int mb200_mass_matrix(mb200_env* e, float* M_dev, void* stream) {
   if (!e || !M_dev) return fail("mb200_mass_matrix: NULL argument");
   CUDA_OK(cudaSetDevice(e->device));
   const LaunchDims d = {grid_for(e), e->warps * 32, e->smem, (cudaStream_t)stream};
-  ops_of(e)->debug(d, e->n, e->phys, e->state, 0, nullptr, M_dev);
+  e->ops->debug(d, e->n, e->phys, e->state, 0, nullptr, M_dev);
   e->launches++;
   CUDA_OK(cudaGetLastError());
   return 0;
@@ -657,72 +585,46 @@ int mb200_inverse_dynamics(mb200_env* e, const float* acc_dev, float* tau_dev, v
   p.lin_damping = 0.0f;  // calculateInverseDynamics has no velocity-damping term
   p.ang_damping = 0.0f;
   const LaunchDims d = {grid_for(e), e->warps * 32, e->smem, (cudaStream_t)stream};
-  ops_of(e)->debug(d, e->n, p, e->state, 1, acc_dev, tau_dev);
+  e->ops->debug(d, e->n, p, e->state, 1, acc_dev, tau_dev);
   e->launches++;
   CUDA_OK(cudaGetLastError());
   return 0;
 }
 
-static int set_record_int(mb200_env* e, int field, const float* values, int count, float scalar) {
+// mb200_set_param (values == nullptr: `scalar` for every env) and mb200_set_param_array: one of the env's
+// MbKindOps::params, checked, into its int record field
+static int set_param(mb200_env* e, const char* key, const float* values, int count, float scalar) {
+  CUDA_OK(cudaSetDevice(e->device));
+  const MbParam* prm = e->ops->params;
+  while (prm->key && strcmp(prm->key, key) != 0) ++prm;
+  if (!prm->key) return fail(std::string("mb200_set_param: unknown key '") + key + "' for this env");
+  const float first = values ? values[0] : scalar;
+  if (prm->check)
+    for (int i = 0; i < (values ? count : 1); ++i)
+      if (const char* err = prm->check(values ? values[i] : scalar, first)) return fail(err);
+  if (prm->variant) e->ops = find_kind(e->ops->env_id, prm->variant(first));
+  if (!values && prm->boolean) scalar = scalar != 0.0f;
   CUDA_OK(cudaDeviceSynchronize());
   const size_t n = (size_t)e->n_pad;
   float* rec = (float*)malloc(n * e->rec_stride * sizeof(float));
   if (!rec) return fail("mb200_set_param: host allocation failed");
   CUDA_OK(cudaMemcpy(rec, e->rec, n * e->rec_stride * sizeof(float), cudaMemcpyDeviceToHost));
-  for (size_t i = 0; i < n; ++i) {
-    const float v = values ? values[i % (size_t)count] : scalar;
-    reinterpret_cast<int*>(rec + i * e->rec_stride)[field] = (int)v;
-  }
+  for (size_t i = 0; i < n; ++i)
+    reinterpret_cast<int*>(rec + i * e->rec_stride)[prm->field] = (int)(values ? values[i % (size_t)count] : scalar);
   CUDA_OK(cudaMemcpy(e->rec, rec, n * e->rec_stride * sizeof(float), cudaMemcpyHostToDevice));
   free(rec);
   return 0;
 }
 
-static int param_field(mb200_env* e, const char* key, float lo, float hi, const float* values, int count, float scalar,
-                       int* field) {
-  if (strcmp(key, "eval_mode") == 0 && custom_family(e->kind)) { *field = ER_EVAL; return 0; }
-  if (strcmp(key, "curriculum") == 0 && stepper_family(e->kind)) {
-    for (int i = 0; i < (values ? count : 1); ++i) {
-      const float v = values ? values[i] : scalar;
-      if (!(v >= 0.0f && v <= 9.0f)) return fail("mb200_set_param: curriculum must be in [0, 9]");
-    }
-    *field = ES_CURRIC;
-    return 0;
-  }
-  if (strcmp(key, "plank_class") == 0 && stepper_family(e->kind)) {
-    for (int i = 0; i < (values ? count : 1); ++i) {
-      const float v = values ? values[i] : scalar;
-      if (!(v == 0.0f || v == 1.0f || v == 2.0f))
-        return fail("mb200_set_param: plank_class must be 0 (LargePlank), 1 (Plank) or 2 (Pillar)");
-      // Pillar runs its own kernel instantiation: the whole batch or none of it
-      if ((v == 2.0f) != ((values ? values[0] : scalar) == 2.0f))
-        return fail("mb200_set_param: plank_class 2 (Pillar) cannot be mixed with other classes in one batch");
-    }
-    *field = ES_PLANK_CLASS;
-    return 0;
-  }
-  if (strcmp(key, "random_reward") == 0 && stepper_family(e->kind)) { *field = ES_RANDOM_REWARD; return 0; }
-  (void)lo; (void)hi;
-  return fail(std::string("mb200_set_param: unknown key '") + key + "' for this env");
-}
-
 int mb200_set_param(mb200_env* e, const char* key, float value) {
   if (!e || !key) return fail("mb200_set_param: NULL argument");
-  CUDA_OK(cudaSetDevice(e->device));
-  int field = 0;
-  if (param_field(e, key, 0, 0, nullptr, 0, value, &field)) return -1;
-  if (field == ES_PLANK_CLASS && stepper_family(e->kind)) e->pillar = value == 2.0f;
-  return set_record_int(e, field, nullptr, 0, field == ER_EVAL && custom_family(e->kind) ? (value != 0.0f) : value);
+  return set_param(e, key, nullptr, 0, value);
 }
 
 int mb200_set_param_array(mb200_env* e, const char* key, const float* values_host, int count) {
   if (!e || !key || !values_host) return fail("mb200_set_param_array: NULL argument");
   if (count != e->n) return fail("mb200_set_param_array: count must equal the number of envs");
-  CUDA_OK(cudaSetDevice(e->device));
-  int field = 0;
-  if (param_field(e, key, 0, 0, values_host, count, 0.0f, &field)) return -1;
-  if (field == ES_PLANK_CLASS && stepper_family(e->kind)) e->pillar = values_host[0] == 2.0f;
-  return set_record_int(e, field, values_host, count, 0.0f);
+  return set_param(e, key, values_host, count, 0.0f);
 }
 
 int mb200_stats(mb200_env* e, double out[8], int reset) {

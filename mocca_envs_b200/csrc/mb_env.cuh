@@ -68,6 +68,38 @@ enum {  // Walker3DStepperEnv additions (env_locomotion.py:330-840)
   ES_TERRAIN = 68,    // [20][6] x y z phi x_tilt y_tilt
 };
 
+// ---- physics parameters (host): the reference's Bullet world.  P is mb200_physics (include/mocca_b200.h) or
+// MbPhysics, which carries the same public fields.
+template <class P> inline void mb_default_physics(P* p) {
+  p->dt = 1.0f / 240.0f; p->substeps = 4; p->iterations = 5; p->gravity = 9.8f; p->erp_contact = 0.9f;
+  p->erp_joint = 0.2f; p->linear_slop = 1e-5f; p->lin_damping = 0.04f; p->ang_damping = 0.04f;
+  p->max_coord_vel = 100.0f; p->limit_max_impulse = 100.0f; p->split_threshold = -0.04f;
+  p->residual_threshold = 1e-7f; p->ground_friction = 0.8f; p->has_ground = 1; p->self_collision = 1;
+  p->warmstart = 0.0f;
+}
+// public parameters -> the solver's; the obstacle contacts start out like the ground's (an env's fix_physics may
+// change them)
+template <class P> inline void mb_to_internal(const P& p, MbPhysics* q) {
+  q->dt = p.dt; q->substeps = p.substeps; q->iterations = p.iterations; q->gravity = p.gravity;
+  q->erp_contact = p.erp_contact; q->erp_joint = p.erp_joint; q->linear_slop = p.linear_slop;
+  q->lin_damping = p.lin_damping; q->ang_damping = p.ang_damping; q->max_coord_vel = p.max_coord_vel;
+  q->limit_max_impulse = p.limit_max_impulse; q->split_threshold = p.split_threshold;
+  q->residual_threshold = p.residual_threshold; q->ground_friction = p.ground_friction; q->has_ground = p.has_ground;
+  q->box_friction = 1.0f; q->box_erp = p.erp_contact; q->box_cfm = 0.0f; q->bar_friction = 0.5f;
+  q->self_collision = p.self_collision;
+  q->warmstart = p.warmstart > 0.0f ? p.warmstart : 0.0f;
+}
+
+// A key mb200_set_param accepts for an env (Env::PARAMS, ended by a null key): the int record field it sets to
+// (int)value for every env.
+struct MbParam {
+  const char* key;
+  int field;
+  bool boolean;                                // the scalar setter stores value != 0
+  const char* (*check)(float v, float first);  // error for value v of a batch whose first value is `first`, or null
+  const char* (*variant)(float first);         // the kernel variant ("" / "pillar") the batch's values select, or null
+};
+
 struct MbStats {  // per-device accumulators, all-reduced across ranks by the host (NCCL) when asked
   unsigned long long episodes;
   unsigned long long steps_reached_sum;  // info["steps_reached"] summed over finished episodes (Stepper, Monkey)
@@ -165,6 +197,45 @@ MB_HD void mb_step_epilogue(typename Env::Mem& S, const MbPhysics& P, float* rec
       if (l == 0) mb_stat_add(&stats->nonfinite, 1ull);
     MB_END
   }
+}
+
+// One stepSimulation of an env: the joint torques tau (nullptr = zero) held over the substeps, the static obstacles of
+// its record.  `points` (nullptr = off) receives the contact points of the last collision pass (what getContactPoints
+// reports after stepSimulation).  Returns the constraint rows; *contacts = the contacts of the last pass.
+template <class Env>
+MB_HD int mb_physics_step(typename Env::Mem& S, const MbPhysics& P, float* state, const float* rec, const float* tau,
+                          float* points, int* contacts) {
+  typedef typename Env::Model M;
+  Env::load_state(S, state);
+  MB_LANES(l)
+    if (l < M::NJ) S.tau[l] = tau ? tau[l] : 0.0f;
+  MB_END
+  int rows = 0, nc = 0, overflow = 0;
+  typename Sim<M>::LaneConst C;
+  Sim<M>::init_lane_const(C);
+#pragma unroll 1
+  for (int k = 0; k < P.substeps; ++k) {
+    Env::load_obstacles(S, rec);
+    rows += Sim<M>::template substep<Env::OBST>(S, P, C, &nc, &overflow, k,
+                                                points && k == P.substeps - 1 ? points : nullptr);
+  }
+  Env::store_state(S, state);
+  *contacts = nc;
+  return rows;
+}
+
+// The mass matrix (S.L, read with mb_Lget) and S.rhs = -bias with zero applied torque, at `state`
+template <class Env> MB_HD void mb_mass_matrix(typename Env::Mem& S, const MbPhysics& P, const float* state) {
+  typedef typename Env::Model M;
+  Env::load_state(S, state);
+  MB_LANES(l)
+    S.tau[l] = 0.0f;
+  MB_END
+  typename Sim<M>::LaneConst C;
+  Sim<M>::init_lane_const(C);
+  Sim<M>::kinematics(S, P, C, true);
+  Sim<M>::bodies(S, P);
+  Sim<M>::mass_matrix_and_rhs(S);
 }
 
 // ------------------------------------------------------------------------------------------------ MT19937
@@ -273,6 +344,11 @@ template <class M> struct W3DEnv {
   typedef M Model;
   enum { NJ = M::NJ, NU = M::NU, OBS = 6 + 2 * M::NJ + M::NFEET + 2, ROBOT_OBS = 6 + 2 * M::NJ + M::NFEET,
          REC_STRIDE = MB_REC_STRIDE, OBST = 0, ACT = M::NJ, INFO_FIELD = -1, CREDIT_STEPS_REACHED = 0 };
+  // the env's kind configuration (host): its own public physics defaults, what it fixes after the caller's
+  // parameters, and the keys of mb200_set_param
+  template <class P> static void default_physics(P&) {}
+  static void fix_physics(MbPhysics&) {}
+  static constexpr MbParam PARAMS[] = {{"eval_mode", ER_EVAL, true, nullptr, nullptr}, {}};
   MB_HD static void load_obstacles(WarpMem<M>&, const float*) {}
 
   // HBM <-> shared
@@ -544,6 +620,33 @@ template <class M, bool PILLAR = false> struct StepperEnv {
   enum { NJ = M::NJ, NU = M::NU, ROBOT_OBS = 6 + 2 * M::NJ + M::NFEET, OBS = ROBOT_OBS + 15, NSTEPS = 20,
          REC_STRIDE = MB_REC_STRIDE_STEPPER, OBST = PILLAR ? MB_OBST_CYLS : MB_OBST_BOXES, ACT = M::NJ,
          INFO_FIELD = ES_STEPS_REACHED, CREDIT_STEPS_REACHED = 1 };
+  template <class P> static void default_physics(P&) {}
+  // remove_ground=True (env_locomotion.py:359); planks: lateralFriction 1.0, contactStiffness 30000, contactDamping
+  // 1000 (bullet_objects.py:64-72) -> per-contact erp / cfm (SURVEY App. B.4); Bullet sums both bodies' contact
+  // damping and a link's default is 0.1
+  static void fix_physics(MbPhysics& p) {
+    p.has_ground = 0;
+    const float kp = 30000.0f, kd = 1000.0f + 0.1f, denom = p.dt * kp + kd;
+    p.box_friction = 1.0f;
+    p.box_erp = p.dt * kp / denom;
+    p.box_cfm = 1.0f / denom;
+  }
+  static const char* check_curriculum(float v, float) {
+    return v >= 0.0f && v <= 9.0f ? nullptr : "mb200_set_param: curriculum must be in [0, 9]";
+  }
+  static const char* check_plank_class(float v, float first) {
+    if (!(v == 0.0f || v == 1.0f || v == 2.0f))
+      return "mb200_set_param: plank_class must be 0 (LargePlank), 1 (Plank) or 2 (Pillar)";
+    // Pillar runs its own kernel instantiation: the whole batch or none of it
+    if ((v == 2.0f) != (first == 2.0f))
+      return "mb200_set_param: plank_class 2 (Pillar) cannot be mixed with other classes in one batch";
+    return nullptr;
+  }
+  static const char* plank_variant(float first) { return first == 2.0f ? "pillar" : ""; }
+  static constexpr MbParam PARAMS[] = {{"curriculum", ES_CURRIC, false, check_curriculum, nullptr},
+                                       {"plank_class", ES_PLANK_CLASS, false, check_plank_class, plank_variant},
+                                       {"random_reward", ES_RANDOM_REWARD, false, nullptr, nullptr},
+                                       {}};
   MB_HD static void load_obstacles(Mem& S, const float* rec) { load_boxes(S, rec); }
   MB_HD static void load_state(Mem& S, const float* st) { B_::load_state(S, st); }
   MB_HD static void store_state(const Mem& S, float* st) { B_::store_state(S, st); }
@@ -872,6 +975,9 @@ template <class M> struct MonkeyEnv {
   enum { NJ = M::NJ, NU = M::NU, ROBOT_OBS = 6 + 2 * M::NJ + M::NFEET, OBS = ROBOT_OBS + 15, NSTEPS = 32, NBARS = 4,
          REC_STRIDE = MB_REC_STRIDE_MONKEY, OBST = MB_OBST_BARS, ACT = M::NJ, INFO_FIELD = -1,
          CREDIT_STEPS_REACHED = 1 };
+  template <class P> static void default_physics(P&) {}
+  static void fix_physics(MbPhysics&) {}
+  static constexpr MbParam PARAMS[] = {{}};
   MB_HD static void load_obstacles(Mem& S, const float* rec) { load_bars(S, rec); }
   MB_HD static void load_state(Mem& S, const float* st) { B_::load_state(S, st); }
   MB_HD static void store_state(const Mem& S, float* st) { B_::store_state(S, st); }
@@ -1170,7 +1276,16 @@ template <class M> struct CassieEnv {
   MB_HD static void load_obstacles(Mem&, const float*) {}
   MB_HD static void load_state(Mem& S, const float* st) { B_::load_state(S, st); }
   MB_HD static void store_state(const Mem& S, float* st) { B_::store_state(S, st); }
-  MB_HD static float control_step() { return 0.03f; }  // env_cassie.py:287
+  static constexpr float CONTROL_STEP = 0.03f;  // env_cassie.py:287
+  MB_HD static float control_step() { return CONTROL_STEP; }
+  // sim_frame_skip 1 (env_cassie.py:287-289, env_base.py:81): one stepSimulation = one substep, LLC_FRAME_SKIP of them
+  // per env step
+  template <class P> static void default_physics(P& p) {
+    p.dt = CONTROL_STEP / LLC_FRAME_SKIP;
+    p.substeps = 1;
+  }
+  static void fix_physics(MbPhysics&) {}
+  static constexpr MbParam PARAMS[] = {{}};
 
   // Joint.current_relative_position + to_radians (bullet_utils.py:212-215, env_cassie.py:204-212): lane k < 14
   MB_HD static float rad_angle(const Mem& S, int k, float* nrm_out) {

@@ -20,6 +20,7 @@
 #define MB_SYNC 1
 #endif
 
+#include "../../include/mocca_b200.h"
 #include "mb_env.cuh"
 
 struct StepArgs {
@@ -65,6 +66,9 @@ struct MbKindOps {
   const char* variant;  // "" or "pillar"
   int obs_dim, act_dim, rec_stride, nj, warps, info_field;
   size_t smem_per_env;
+  void (*default_physics)(mb200_physics&);  // the env's own public defaults (Env::default_physics)
+  void (*fix_physics)(MbPhysics&);           // applied after the caller's parameters (Env::fix_physics)
+  const MbParam* params;                     // the keys mb200_set_param accepts (Env::PARAMS)
   cudaError_t (*prepare)(void);  // shared-memory opt-in of every kernel of the kind
   void (*step)(const StepArgs&, bool host, const LaunchDims&);
   void (*reset)(const LaunchDims&, int n, const MbPhysics&, float* state, float* rec, uint32_t* mt, const uint8_t* mask,
@@ -150,26 +154,14 @@ __device__ __forceinline__ void physics_body(int n, const MbPhysics& phys, float
   const int warp = threadIdx.x >> 5;
   const int env = blockIdx.x * MB_WARPS + warp;
   const bool tail = env >= n;  // pad env: steps with zero torque, outputs discarded
-  typedef typename Env::Model EM;
   typename Env::Mem& S = reinterpret_cast<typename Env::Mem*>(smem_raw)[warp];
   if ((threadIdx.x & 31) == 0) S.warm = warm ? warm + (size_t)env * MB_NWARM : nullptr;
   __syncwarp();
-  Env::load_state(S, state + (size_t)env * MB_STATE_STRIDE);
-  MB_LANES(l)
-    if (l < EM::NJ) S.tau[l] = tail ? 0.0f : tau[(size_t)env * EM::NJ + l];
-  MB_END
-  int rows = 0, nc = 0, overflow = 0;
-  typename Sim<EM>::LaneConst C;
-  Sim<EM>::init_lane_const(C);
-#pragma unroll 1
-  for (int k = 0; k < phys.substeps; ++k) {
-    Env::load_obstacles(S, rec + (size_t)env * Env::REC_STRIDE);
-    // the contact points of the LAST collision pass (what getContactPoints reports after stepSimulation)
-    float* pts = points_out && !tail && k == phys.substeps - 1
-                     ? points_out + (size_t)env * MB_MAXC * MB_POINT_WIDTH : nullptr;
-    rows += Sim<EM>::template substep<Env::OBST>(S, phys, C, &nc, &overflow, k, pts);
-  }
-  Env::store_state(S, state + (size_t)env * MB_STATE_STRIDE);
+  int nc;
+  const int rows = mb_physics_step<Env>(
+      S, phys, state + (size_t)env * MB_STATE_STRIDE, rec + (size_t)env * Env::REC_STRIDE,
+      tail ? nullptr : tau + (size_t)env * Env::Model::NJ,
+      points_out && !tail ? points_out + (size_t)env * MB_MAXC * MB_POINT_WIDTH : nullptr, &nc);
   if (tail) return;
   if ((threadIdx.x & 31) == 0) {
     if (rows_out) rows_out[env] = rows;
@@ -190,15 +182,7 @@ __device__ __forceinline__ void dynamics_debug_body(int n, const MbPhysics& phys
   const int NU = EM::NU;
   if ((threadIdx.x & 31) == 0) S.warm = nullptr;
   __syncwarp();
-  Env::load_state(S, state + (size_t)env * MB_STATE_STRIDE);
-  MB_LANES(l)
-    S.tau[l] = 0.0f;
-  MB_END
-  typename Sim<EM>::LaneConst C;
-  Sim<EM>::init_lane_const(C);
-  Sim<EM>::kinematics(S, phys, C, true);
-  Sim<EM>::bodies(S, phys);
-  Sim<EM>::mass_matrix_and_rhs(S);
+  mb_mass_matrix<Env>(S, phys, state + (size_t)env * MB_STATE_STRIDE);
   MB_LANES(l)
     if (l < NU) {
       if (mode == 0) {
@@ -261,6 +245,8 @@ __device__ __forceinline__ void dynamics_debug_body(int n, const MbPhysics& phys
     k_dynamics_debug_##ID<<<d.grid, d.threads, d.smem, d.stream>>>(n, p, state, mode, acc, out);                      \
   }                                                                                                                   \
   extern const MbKindOps mb_kind_##ID = {ENV_ID, VARIANT, ENV::OBS, ENV::ACT, ENV::REC_STRIDE, ENV::Model::NJ,       \
-                                         WARPS, ENV::INFO_FIELD, sizeof(typename ENV::Mem), prepare_##ID,            \
+                                         WARPS, ENV::INFO_FIELD, sizeof(typename ENV::Mem),                          \
+                                         ENV::template default_physics<mb200_physics>, ENV::fix_physics, ENV::PARAMS, \
+                                         prepare_##ID,                                                               \
                                          launch_step_##ID, launch_reset_##ID, launch_physics_##ID,                    \
                                          launch_debug_##ID};

@@ -53,6 +53,15 @@ def _ptr(t):
     return None if t is None else C.c_void_p(t.data_ptr())
 
 
+def _unsupported(message=None):
+    """A trainer-facing method the reference env does not have: it raises AttributeError(message), or does nothing
+    when there is no message."""
+    def method(self, *args):
+        if message is not None:
+            raise AttributeError(message)
+    return method
+
+
 class Walker3DCustomVecEnv:
     """Batched Walker3DCustomEnv-v0; also the base class of the other batched envs (env_id selects the kernels)."""
 
@@ -297,25 +306,35 @@ class Walker3DCustomVecEnv:
         raise AttributeError("set_robot_params: the reference calls the undefined robot.calc_torque_limits() "
                              "(env_base.py:114); no robot parameter can be changed after construction")
 
+    # the env credits info["steps_reached"] to the statistics at every episode end (the kernel's CREDIT_STEPS_REACHED)
+    reports_steps_reached = False
+
     def stats(self, reset=False) -> dict:
         out = (C.c_double * 8)()
         _lib.check(self._L.mb200_stats(self._h, out, int(reset)))
-        return {"episodes": out[0], "return_sum": out[1], "length_sum": out[2], "nonfinite": out[3],
-                "overflow": out[4]}
+        d = {"episodes": out[0], "return_sum": out[1], "length_sum": out[2], "nonfinite": out[3], "overflow": out[4]}
+        if self.reports_steps_reached:
+            d["steps_reached_sum"] = out[5]
+        return d
 
     def launch_count(self) -> int:
         return int(self._L.mb200_launch_count(self._h))
 
+    # observation entries past the robot state that mirroring negates: the target's lateral offset
+    mirror_neg_targets = (0,)
+
     def get_mirror_indices(self):
-        """Walker3DCustomEnv.get_mirror_indices (env_locomotion.py:224-282) -- static index tables."""
+        """Walker3DCustomEnv / Walker3DStepperEnv.get_mirror_indices (env_locomotion.py:224-282,761-840) -- static
+        index tables."""
         A = self.act_dim
         right_j = np.array(self.table["right_joint_indices"], dtype=np.int64)
         left_j = np.array(self.table["left_joint_indices"], dtype=np.int64)
         neg_j = np.array(self.table["negation_joint_indices"], dtype=np.int64)
         nfeet = len(self.table["foot_links"])
+        robot_obs = 6 + 2 * A + nfeet
         right = np.concatenate((right_j + 6, right_j + 6 + A, [6 + 2 * A + 2 * i for i in range(nfeet // 2)]))
         left = np.concatenate((left_j + 6, left_j + 6 + A, [6 + 2 * A + 2 * i + 1 for i in range(nfeet // 2)]))
-        neg_obs = np.concatenate(([2, 4], 6 + neg_j, 6 + neg_j + A, [6 + 2 * A + nfeet]))
+        neg_obs = np.concatenate(([2, 4], 6 + neg_j, 6 + neg_j + A, robot_obs + np.array(self.mirror_neg_targets)))
         return neg_obs, right, left, neg_j, right_j, left_j
 
 
@@ -327,6 +346,10 @@ class Walker3DStepperVecEnv(Walker3DCustomVecEnv):
     ES_NEXT, ES_CURRIC, ES_STEPS_REACHED, ES_TERRAIN = 22, 27, 31, 68
     max_curriculum = 9
     curriculum = 0  # env_locomotion.py:363
+    reports_steps_reached = True
+    # the lateral offset and the x tilt of each of the three step targets (env_locomotion.py:761-840)
+    mirror_neg_targets = (0, 3, 5, 8, 10, 13)
+    evaluation_mode = _unsupported("Walker3DStepperEnv has no evaluation_mode (reference: only Walker3DCustomEnv)")
 
     def __init__(self, num_envs: int, device="cuda:0", seed: int | None = None, physics: dict | None = None,
                  return_final_obs: bool = False, random_reward: bool = False, plank_class: str | None = None):
@@ -362,9 +385,6 @@ class Walker3DStepperVecEnv(Walker3DCustomVecEnv):
                                                          len(arr)))
                 self.curriculum = arr.astype(np.int64)
 
-    def evaluation_mode(self):
-        raise AttributeError("Walker3DStepperEnv has no evaluation_mode (reference: only Walker3DCustomEnv)")
-
     def _host_params(self) -> dict:
         cur = self.curriculum
         return {"curriculum": cur.tolist() if isinstance(cur, np.ndarray) else int(cur),
@@ -389,26 +409,6 @@ class Walker3DStepperVecEnv(Walker3DCustomVecEnv):
     def terrain_info(self) -> torch.Tensor:
         return self.get_record()[:, self.ES_TERRAIN:self.ES_TERRAIN + 120].reshape(self.num_envs, 20, 6)
 
-    def stats(self, reset=False) -> dict:
-        out = (C.c_double * 8)()
-        _lib.check(self._L.mb200_stats(self._h, out, int(reset)))
-        return {"episodes": out[0], "return_sum": out[1], "length_sum": out[2], "nonfinite": out[3],
-                "overflow": out[4], "steps_reached_sum": out[5]}
-
-    def get_mirror_indices(self):
-        """Walker3DStepperEnv.get_mirror_indices (env_locomotion.py:761-840)."""
-        A = self.act_dim
-        right_j = np.array(self.table["right_joint_indices"], dtype=np.int64)
-        left_j = np.array(self.table["left_joint_indices"], dtype=np.int64)
-        neg_j = np.array(self.table["negation_joint_indices"], dtype=np.int64)
-        nfeet = len(self.table["foot_links"])
-        robot_obs = 6 + 2 * A + nfeet
-        right = np.concatenate((6 + right_j, 6 + right_j + A, [6 + 2 * A + 2 * i for i in range(nfeet // 2)]))
-        left = np.concatenate((6 + left_j, 6 + left_j + A, [6 + 2 * A + 2 * i + 1 for i in range(nfeet // 2)]))
-        robot_neg = np.concatenate(([2, 4], 6 + neg_j, 6 + neg_j + A))
-        steps_neg = np.array([(i * 5 + 0, i * 5 + 3) for i in range(3)], dtype=np.int64).flatten()
-        neg_obs = np.concatenate((robot_neg, steps_neg + robot_obs))
-        return neg_obs, right, left, neg_j, right_j, left_j
 
 
 class Child3DCustomVecEnv(Walker3DCustomVecEnv):
@@ -454,30 +454,19 @@ class Monkey3DCustomVecEnv(Walker3DCustomVecEnv):
     env_id = MONKEY_ID
     model = "monkey3d"
     EM_NEXT, EM_FREEFALL, EM_TIMESTEP, EM_SWING, EM_PIVOT, EM_BAR, EM_TERRAIN = 22, 23, 24, 25, 26, 32, 64
+    reports_steps_reached = True
+    evaluation_mode = _unsupported("Monkey3DCustomEnv has no evaluation_mode (reference: only Walker3DCustomEnv)")
+    set_env_params = _unsupported()
+    get_mirror_indices = _unsupported("Monkey3DCustomEnv defines no get_mirror_indices in the reference")
 
     def _action_space(self):  # env_locomotion.py:1179-1181: unbounded torque space
         return Box(-np.inf * np.ones(self.act_dim), np.inf * np.ones(self.act_dim))
-
-    def evaluation_mode(self):
-        raise AttributeError("Monkey3DCustomEnv has no evaluation_mode (reference: only Walker3DCustomEnv)")
-
-    def set_env_params(self, params: dict):
-        pass
 
     def terrain_info(self) -> torch.Tensor:
         return self.get_record()[:, self.EM_TERRAIN:self.EM_TERRAIN + 128].reshape(self.num_envs, 32, 4)
 
     def next_step_index(self) -> torch.Tensor:
         return self.get_record()[:, self.EM_NEXT].contiguous().view(torch.int32)
-
-    def stats(self, reset=False) -> dict:
-        out = (C.c_double * 8)()
-        _lib.check(self._L.mb200_stats(self._h, out, int(reset)))
-        return {"episodes": out[0], "return_sum": out[1], "length_sum": out[2], "nonfinite": out[3],
-                "overflow": out[4], "steps_reached_sum": out[5]}
-
-    def get_mirror_indices(self):
-        raise AttributeError("Monkey3DCustomEnv defines no get_mirror_indices in the reference")
 
 
 class CassieVecEnv(Walker3DCustomVecEnv):
@@ -492,15 +481,9 @@ class CassieVecEnv(Walker3DCustomVecEnv):
     llc_frame_skip = 50  # env_cassie.py:288
     sim_frame_skip = 1  # env_cassie.py:289
     EC_POTENTIAL, EC_JVEL = 22, 32
-
-    def evaluation_mode(self):
-        raise AttributeError("CassieEnv has no evaluation_mode")
-
-    def set_env_params(self, params: dict):
-        pass
-
-    def get_mirror_indices(self):
-        raise AttributeError("CassieEnv-v0 defines no get_mirror_indices in the reference")
+    evaluation_mode = _unsupported("CassieEnv has no evaluation_mode")
+    set_env_params = _unsupported()
+    get_mirror_indices = _unsupported("CassieEnv-v0 defines no get_mirror_indices in the reference")
 
     def rewards_info(self, obs_rew: torch.Tensor | None = None) -> dict:
         """The reference returns the reward terms as ``info`` (env_cassie.py:479): AliveRew = +2 / -1,
@@ -588,14 +571,12 @@ class Walker3DStepperEnv(Walker3DCustomEnv):
 
     vec_class = Walker3DStepperVecEnv
     vec_kwargs = ("random_reward", "plank_class")  # env_locomotion.py:355-357
+    evaluation_mode = _unsupported("Walker3DStepperEnv has no evaluation_mode")
 
     def _extra_info(self, info):
         sr = int(self.vec.steps_reached()[0].item())
         if sr >= 0:
             info["steps_reached"] = sr
-
-    def evaluation_mode(self):
-        raise AttributeError("Walker3DStepperEnv has no evaluation_mode")
 
 
 class Child3DCustomEnv(Walker3DCustomEnv):
@@ -628,6 +609,7 @@ class Monkey3DCustomEnv(Walker3DCustomEnv):
     and this facade mirrors the visible side effect."""
 
     vec_class = Monkey3DCustomVecEnv
+    evaluation_mode = _unsupported("Monkey3DCustomEnv has no evaluation_mode")
 
     def step(self, action):
         rec = self.vec.get_record()[0]
@@ -639,22 +621,17 @@ class Monkey3DCustomEnv(Walker3DCustomEnv):
             action[17 if pivot == 0 else 22] = -1
         return out
 
-    def evaluation_mode(self):
-        raise AttributeError("Monkey3DCustomEnv has no evaluation_mode")
-
 
 class CassieEnv(Walker3DCustomEnv):
     """gym-protocol facade of CassieEnv-v0; ``info`` carries the reward terms like the reference."""
 
     vec_class = CassieVecEnv
+    evaluation_mode = _unsupported("CassieEnv has no evaluation_mode")
 
     def _extra_info(self, info):
         r = self.vec.rewards_info()
         info["AliveRew"] = float(r["AliveRew"][0].item())
         info["ProgressRew"] = float(r["ProgressRew"][0].item())
-
-    def evaluation_mode(self):
-        raise AttributeError("CassieEnv has no evaluation_mode")
 
 
 _REGISTRY = {ENV_ID: (Walker3DCustomEnv, Walker3DCustomVecEnv), STEPPER_ID: (Walker3DStepperEnv, Walker3DStepperVecEnv),

@@ -39,18 +39,9 @@ def lib():
     return _lib
 
 
-def _phys(fn):
-    p = Phys()
-    getattr(lib(), fn)(C.byref(p))
-    return p
-
-
 def default_phys():
-    return _phys("emu_default_phys")
-
-
-def cassie_phys():
-    return _phys("emu_cassie_phys")
+    """The plain reference physics (Walker3DCustomEnv has no physics of its own)."""
+    return EmuW3D.phys()
 
 
 def _fp(a):
@@ -59,15 +50,21 @@ def _fp(a):
 
 class EmuEnv:
     """One env through the emulated kernel source: emu_<prefix>_* in emu.cpp (record layout: ER_* and the kind's
-    additions in mb_env.cuh).  A subclass per env kind names its prefix, dimensions and physics defaults."""
+    additions in mb_env.cuh).  A subclass per env kind names its prefix and dimensions."""
 
     prefix = None
     obs_dim = act_dim = n_dof = None
-    phys_fn = "emu_default_phys"  # the kind's physics defaults (as mb200_create sets them)
     aliased = 1  # ER_ALIASED: the robot draws from the env stream until the env is re-seeded
 
+    @classmethod
+    def phys(cls):
+        """The kind's physics as mb200_create sets them when the caller passes none."""
+        p = Phys()
+        getattr(lib(), "emu_%s_phys" % cls.prefix)(C.byref(p))
+        return p
+
     def __init__(self, mt_state=None, phys=None):
-        self.p = phys or _phys(self.phys_fn)
+        self.p = phys or self.phys()
         self.state = np.zeros(64, dtype=np.float32)
         self.rec = np.zeros(self._call("rec_stride"), dtype=np.float32)
         self.rec.view(np.int32)[11] = self.aliased
@@ -145,7 +142,6 @@ class EmuStepper(EmuEnv):
 
     prefix = "stepper"
     obs_dim, act_dim, n_dof = 65, 21, 21
-    phys_fn = "emu_stepper_phys"
 
     ES_NEXT, ES_COUNT, ES_STOP, ES_SETSTOP, ES_TIMESTEP, ES_CURRIC, ES_PLANKIDX, ES_STEPS = 22, 23, 24, 25, 26, 27, 28, 31
     ES_BOX, ES_TERRAIN = 32, 68
@@ -186,7 +182,6 @@ class EmuCassie(EmuEnv):
 
     prefix = "cassie"
     obs_dim, act_dim, n_dof = 36, 10, 18
-    phys_fn = "emu_cassie_phys"
     aliased = 0
 
     EC_POTENTIAL, EC_JVEL = 22, 32
