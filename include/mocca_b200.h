@@ -133,8 +133,13 @@ int mb200_step_physics(mb200_env* env, const float* tau_dev, int* rows_dev, int*
  * for feet_contact; bullet_utils.py:177-181): the contact points of the LAST collision pass with the normal impulse the
  * solver applied to each.  points_dev is [n][mb200_max_contact_points()][mb200_contact_point_width()] float32:
  * {world position on the robot link (3), contact normal on the partner pointing to the link (3), distance, normal
- * impulse, robot link index (-1 = base, -2 = unused slot), partner (0 ground plane, 10 + k plank box k, 20 + k bar k,
- * 1000 + p self-collision pair p)}.  Parity / golden-vector entry point; the env step kernels do not produce it. */
+ * impulse, robot link index, partner}.  The link index is the dof index of the movable frame that carries the geom:
+ * a fixed link is folded into its nearest movable ancestor, -1 is the base and -2 an unused slot (so it is not the URDF
+ * link index pybullet reports when the model has fixed links).  The partner is 0 for the ground plane, 10 + k for
+ * plank box k (plank k / 2: k even = base box, k odd = cover), 20 + k for bar k and 1000 + p for a self-contact, where
+ * p indexes the env kind's self-collision pair table (the model's "self_pairs", geom A then geom B; the point is on A's
+ * link and the normal points from B to A).  Unused slots are zero apart from their link index.  Parity /
+ * golden-vector entry point; the env step kernels do not produce it. */
 int mb200_max_contact_points(void);
 int mb200_contact_point_width(void);
 int mb200_step_physics_points(mb200_env* env, const float* tau_dev, int* rows_dev, int* contacts_dev, float* points_dev,
