@@ -150,6 +150,23 @@ int mb200_step_physics_points(mb200_env* env, const float* tau_dev, int* rows_de
 int mb200_mass_matrix(mb200_env* env, float* M_dev, void* stream);
 int mb200_inverse_dynamics(mb200_env* env, const float* acc_dev, float* tau_dev, void* stream);
 
+/* A push between two env steps: env i receives the instantaneous linear impulse impulse_dev[i] (N s, world frame) at the
+ * world point point_dev[i], rigidly attached to link link_dev[i] (shapes [n], [n][3], [n][3], device memory).  The
+ * generalised velocity u = [omega_world, v_world, qd] (the coordinates of mb200_mass_matrix) changes by
+ *   du = M(q)^-1 J(point)^T impulse,
+ * then u is clamped to +-max_coord_vel as in every substep.  Positions, quaternion, q, the record, the RNG streams and
+ * the warm-start impulses are untouched; contacts and joint limits do not act at the instant of the push (the next
+ * substep's rows react to the new velocity).  A force F held over one env step is, to first order, the impulse
+ * F * control_step; this is not pybullet.applyExternalForce.  The observation the caller holds is the pre-push one.
+ * Link index: -1 = the base, j = the movable frame of dof j with fixed links folded into their nearest movable ancestor
+ * (the link index of mb200_step_physics_points).  Any other index (e.g. -2), an all-zero impulse or a non-finite
+ * impulse or point leaves that env untouched, bit for bit.
+ * CassieEnv-v0: the response keeps the two achilles-rod loop closures closed: du = M^-1 (J^T impulse - G^T lambda) with
+ * G du = 0 (G = the six point-to-point rows).  Walker2D / Crab2D: the y components of impulse and point are taken as
+ * zero (what the planar root transmits), so the motion stays exactly in the x-z plane. */
+int mb200_apply_impulse(mb200_env* env, const int* link_dev, const float* point_dev, const float* impulse_dev,
+                        void* stream);
+
 /* EnvBase.set_env_params analogue (env_base.py:103-106): "eval_mode" (Walker3DCustomEnv, env_locomotion.py:76-77),
  * "curriculum" 0..9 (Walker3DStepperEnv, env_locomotion.py:362-369; takes effect at the next reset like the
  * reference, whose terrain / gain / terminal height are read in reset() and step()), "random_reward" 0 / 1

@@ -26,7 +26,8 @@ SYMBOLS = [
     "mb200_reset_host", "mb200_info", "mb200_info_host", "mb200_step_physics_points", "mb200_max_contact_points",
     "mb200_contact_point_width", "mb200_warm_width", "mb200_get_warm", "mb200_set_warm",
     "mb200_step", "mb200_step_host", "mb200_get_state", "mb200_set_state", "mb200_get_record", "mb200_set_record",
-    "mb200_rng_words", "mb200_get_rng", "mb200_set_rng", "mb200_step_physics", "mb200_mass_matrix", "mb200_inverse_dynamics", "mb200_set_param",
+    "mb200_rng_words", "mb200_get_rng", "mb200_set_rng", "mb200_step_physics", "mb200_mass_matrix", "mb200_inverse_dynamics",
+    "mb200_apply_impulse", "mb200_set_param",
     "mb200_set_param_array", "mb200_record_stride", "mb200_stats",
     "mb200_launch_count", "mb200_measure_fp32_peak", "mb200_last_error",
 ]
@@ -120,6 +121,7 @@ def lib():
         L.mb200_get_rng.argtypes = [vp, vp]
         L.mb200_set_rng.argtypes = [vp, vp]
         L.mb200_inverse_dynamics.argtypes = [vp, vp, vp, vp]
+        L.mb200_apply_impulse.argtypes = [vp, vp, vp, vp, vp]
         L.mb200_set_param.argtypes = [vp, C.c_char_p, C.c_float]
         L.mb200_set_param_array.argtypes = [vp, C.c_char_p, vp, ip]
         L.mb200_record_stride.argtypes = [vp]

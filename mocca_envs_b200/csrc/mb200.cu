@@ -591,6 +591,17 @@ int mb200_inverse_dynamics(mb200_env* e, const float* acc_dev, float* tau_dev, v
   return 0;
 }
 
+int mb200_apply_impulse(mb200_env* e, const int* link_dev, const float* point_dev, const float* impulse_dev,
+                        void* stream) {
+  if (!e || !link_dev || !point_dev || !impulse_dev) return fail("mb200_apply_impulse: NULL argument");
+  CUDA_OK(cudaSetDevice(e->device));
+  const LaunchDims d = {grid_for(e), e->warps * 32, e->smem, (cudaStream_t)stream};
+  e->ops->impulse(d, e->n, e->phys, e->state, link_dev, point_dev, impulse_dev);
+  e->launches++;
+  CUDA_OK(cudaGetLastError());
+  return 0;
+}
+
 // mb200_set_param (values == nullptr: `scalar` for every env) and mb200_set_param_array: one of the env's
 // MbKindOps::params, checked, into its int record field
 static int set_param(mb200_env* e, const char* key, const float* values, int count, float scalar) {

@@ -238,6 +238,127 @@ template <class Env> MB_HD void mb_mass_matrix(typename Env::Mem& S, const MbPhy
   Sim<M>::mass_matrix_and_rhs(S);
 }
 
+// z -= Y_G (Y_G^T Y_G)^-1 Y_G^T z: the part of the push in z = L du space that would open a loop closure is removed, so
+// that G du = Y_G^T z = 0 afterwards.  g[i] is loop multiplier i's row Y = L^-T G_i^T, lane-indexed (the sum of its two
+// compact parts).  Y_G^T Y_G = G M^-1 G^T exactly, coupling term included (Bullet's PGS denominator drops it; this
+// projection is not a PGS row and needs the exact Gram matrix).  Every lane holds the 6x6 system and solves it alike.
+template <int NG>
+MB_HD void mb_project_loops(const LaneVar<float>* g, LaneVar<float>& z) {
+  float A[NG][NG], b[NG];
+#pragma unroll
+  for (int i = 0; i < NG; ++i) {
+    LaneVar<float> t;
+#pragma unroll
+    for (int j = 0; j <= i; ++j) {
+      MB_LANES(l)
+        t[l] = g[i][l] * g[j][l];
+      MB_END_REG
+      A[i][j] = warp_sum(t);
+    }
+    MB_LANES(l)
+      t[l] = g[i][l] * z[l];
+    MB_END_REG
+    b[i] = warp_sum(t);
+  }
+  // Cholesky A = R R^T in place (lower triangle), then R R^T lambda = b
+#pragma unroll
+  for (int k = 0; k < NG; ++k) {
+    float d = A[k][k];
+#pragma unroll
+    for (int s = 0; s < k; ++s) d -= A[k][s] * A[k][s];
+    const float rinv = d > 0.0f ? 1.0f / sqrtf(d) : 0.0f;  // (a degenerate loop row takes no multiplier)
+    A[k][k] = rinv;
+#pragma unroll
+    for (int i = k + 1; i < NG; ++i) {
+      float v = A[i][k];
+#pragma unroll
+      for (int s = 0; s < k; ++s) v -= A[i][s] * A[k][s];
+      A[i][k] = v * rinv;
+    }
+  }
+#pragma unroll
+  for (int i = 0; i < NG; ++i) {
+#pragma unroll
+    for (int s = 0; s < i; ++s) b[i] -= A[i][s] * b[s];
+    b[i] *= A[i][i];
+  }
+#pragma unroll
+  for (int i = NG - 1; i >= 0; --i) {
+#pragma unroll
+    for (int s = i + 1; s < NG; ++s) b[i] -= A[s][i] * b[s];
+    b[i] *= A[i][i];
+  }
+  MB_LANES(l)
+#pragma unroll
+    for (int i = 0; i < NG; ++i) z[l] = fmaf(-b[i], g[i][l], z[l]);
+  MB_END_REG
+}
+
+// An instantaneous linear impulse (N s, world frame) at the world point `point` rigidly attached to `link` (-1 = the
+// base, j = the movable frame of dof j), between two env steps:  du = M(q)^-1 J(point)^T impulse, u = [omega_w, v_w, qd],
+// clamped to +-max_coord_vel like every velocity update of a substep.  Cassie's loop closures are kept closed
+// (du = M^-1 (J^T impulse - G^T lambda) with G du = 0, mb_project_loops).  Planar models push with the y components of
+// impulse and point set to zero: what their slide-x / slide-z / hinge-y root transmits.  Positions, q and everything
+// outside `state` are untouched; so is the whole env for a link outside [-1, NJ), a zero impulse or a non-finite input.
+// The push is one synthetic contact-normal row through row_build: its Y = L^-T J^T is the push itself in z space.
+template <class Env>
+MB_HD void mb_apply_impulse(typename Env::Mem& S, const MbPhysics& P, float* state, int link, const float* point,
+                            const float* impulse) {
+  typedef typename Env::Model M;
+  typedef Sim<M> Q;
+  float iv[3] = {impulse[0], impulse[1], impulse[2]}, pv[3] = {point[0], point[1], point[2]};
+  if (M::planar_env()) { iv[1] = 0.0f; pv[1] = 0.0f; }
+  const float mag = sqrtf(mb_dot3(iv, iv));
+  bool ok = link >= -1 && link < M::NJ && mag > 0.0f && mb_finite(mag);
+  for (int k = 0; k < 3; ++k) ok = ok && mb_finite(pv[k]);
+  if (!ok) return;
+  Env::load_state(S, state);
+  MB_LANES(l)
+    S.tau[l] = 0.0f;
+  MB_END
+  typename Q::LaneConst C;
+  Q::init_lane_const(C);
+  Q::kinematics(S, P, C, true);
+  Q::loop_pivots(S);  // (reads jR / jp: the rows below overwrite them)
+  Q::bodies(S, P);
+  Q::mass_matrix_and_rhs(S);
+  Q::template factorize<false>(S, C);
+  MB_LANES(l)
+    if (l == 0) {
+      const float inv = 1.0f / mag;
+      for (int k = 0; k < 3; ++k) { S.cP[0][k] = pv[k] - S.pos[k]; S.cn[0][k] = iv[k] * inv; }
+      S.cdist[0] = 0.0f; S.cmu[0] = 0.0f; S.cerp[0] = 0.0f; S.ccfm[0] = 0.0f;
+      S.clink[0] = link; S.cfoot[0] = 0; S.cpartner[0] = 0;
+    }
+  MB_END
+  // rows: the loop closures [0, NLC) (no limit rows), then the push as contact slot 0
+  MB_LANES(l)
+    if (l <= Q::NLC) Q::row_build(S, P, 0, 1, 0, l);
+  MB_END
+  LaneVar<float> z;
+  const unsigned sup = S.rc.r.r_mask[Q::NLC] & MB_ROW_SUP;
+  MB_LANES(l)
+    z[l] = ((sup >> l) & 1u) ? S.w.Yc[Q::NLC][C.tl[l]] * mag : 0.0f;
+  MB_END_REG
+  if constexpr (M::NLOOP > 0) {
+    LaneVar<float> g[Q::NLC / 2];
+#pragma unroll
+    for (int i = 0; i < Q::NLC / 2; ++i) {
+      const unsigned sa = S.rc.r.r_mask[2 * i] & MB_ROW_SUP, sb = S.rc.r.r_mask[2 * i + 1] & MB_ROW_SUP;
+      MB_LANES(l)
+        g[i][l] = (((sa >> l) & 1u) ? S.w.Yc[2 * i][C.tl[l]] : 0.0f) +
+                  (((sb >> l) & 1u) ? S.w.Yc[2 * i + 1][C.tl[l]] : 0.0f);
+      MB_END_REG
+    }
+    mb_project_loops<Q::NLC / 2>(g, z);
+  }
+  Q::template solve_L<false>(S, C, z);
+  MB_LANES(l)
+    if (l < M::NU) S.u[l] = fminf(fmaxf(S.u[l] + z[l], -P.max_coord_vel), P.max_coord_vel);
+  MB_END
+  Env::store_state(S, state);
+}
+
 // ------------------------------------------------------------------------------------------------ MT19937
 // NumPy legacy RandomState stream, warp-cooperative.  mt[0..623] state words, mt[624] position.
 MB_HD void mt_twist(uint32_t* mt) {

@@ -76,6 +76,8 @@ struct MbKindOps {
   void (*physics)(const LaunchDims&, int n, const MbPhysics&, float* state, const float* rec, const float* tau,
                   int* rows_out, int* contacts_out, float* points_out, float* warm);
   void (*debug)(const LaunchDims&, int n, const MbPhysics&, const float* state, int mode, const float* acc, float* out);
+  void (*impulse)(const LaunchDims&, int n, const MbPhysics&, float* state, const int* link, const float* point,
+                  const float* impulse);
 };
 
 template <class Env, bool HOST>
@@ -196,7 +198,22 @@ __device__ __forceinline__ void dynamics_debug_body(int n, const MbPhysics& phys
   MB_END
 }
 
-// One env kind: step (device / host-buffer instantiations), reset, physics-only and debug kernels + its MbKindOps.
+// mb200_apply_impulse: env `env` gets impulse[env] at point[env] on link[env] (mb_apply_impulse); pad envs and envs the
+// push leaves untouched return at once (no CTA barrier on this path)
+template <class Env>
+__device__ __forceinline__ void impulse_body(int n, const MbPhysics& phys, float* state, const int* link,
+                                             const float* point, const float* impulse) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  const int warp = threadIdx.x >> 5;
+  const int env = blockIdx.x * MB_WARPS + warp;
+  if (env >= n) return;
+  typename Env::Mem& S = reinterpret_cast<typename Env::Mem*>(smem_raw)[warp];
+  mb_apply_impulse<Env>(S, phys, state + (size_t)env * MB_STATE_STRIDE, link[env], point + 3 * (size_t)env,
+                        impulse + 3 * (size_t)env);
+}
+
+// One env kind: step (device / host-buffer instantiations), reset, physics-only, debug and impulse kernels + its
+// MbKindOps.
 #define MB_DEFINE_KIND(ID, ENV_ID, VARIANT, ENV, WARPS)                                                               \
   __global__ void __launch_bounds__(WARPS * 32, MB_MINBLOCKS) k_step_##ID(StepArgs a) { step_body<ENV, false>(a); }  \
   __global__ void __launch_bounds__(WARPS * 32, MB_MINBLOCKS) k_step_##ID##_host(StepArgs a) {                       \
@@ -216,6 +233,11 @@ __device__ __forceinline__ void dynamics_debug_body(int n, const MbPhysics& phys
       k_dynamics_debug_##ID(int n, MbPhysics phys, const float* state, int mode, const float* acc, float* out) {     \
     dynamics_debug_body<ENV>(n, phys, state, mode, acc, out);                                                         \
   }                                                                                                                   \
+  __global__ void __launch_bounds__(MB_WARPS_MAX * 32)                                                                \
+      k_apply_impulse_##ID(int n, MbPhysics phys, float* state, const int* link, const float* point,                 \
+                           const float* impulse) {                                                                    \
+    impulse_body<ENV>(n, phys, state, link, point, impulse);                                                          \
+  }                                                                                                                   \
   static cudaError_t prepare_##ID(void) {                                                                             \
     const int bytes = (int)(sizeof(typename ENV::Mem) * WARPS);                                                \
     const cudaFuncAttribute at = cudaFuncAttributeMaxDynamicSharedMemorySize;                                         \
@@ -224,7 +246,8 @@ __device__ __forceinline__ void dynamics_debug_body(int n, const MbPhysics& phys
     if ((e = cudaFuncSetAttribute(k_step_##ID##_host, at, bytes)) != cudaSuccess) return e;                           \
     if ((e = cudaFuncSetAttribute(k_reset_##ID, at, bytes)) != cudaSuccess) return e;                                 \
     if ((e = cudaFuncSetAttribute(k_step_physics_##ID, at, bytes)) != cudaSuccess) return e;                          \
-    return cudaFuncSetAttribute(k_dynamics_debug_##ID, at, bytes);                                                    \
+    if ((e = cudaFuncSetAttribute(k_dynamics_debug_##ID, at, bytes)) != cudaSuccess) return e;                       \
+    return cudaFuncSetAttribute(k_apply_impulse_##ID, at, bytes);                                                     \
   }                                                                                                                   \
   static void launch_step_##ID(const StepArgs& a, bool host, const LaunchDims& d) {                                   \
     if (host) k_step_##ID##_host<<<d.grid, d.threads, d.smem, d.stream>>>(a);                                         \
@@ -244,9 +267,13 @@ __device__ __forceinline__ void dynamics_debug_body(int n, const MbPhysics& phys
                                 const float* acc, float* out) {                                                       \
     k_dynamics_debug_##ID<<<d.grid, d.threads, d.smem, d.stream>>>(n, p, state, mode, acc, out);                      \
   }                                                                                                                   \
+  static void launch_impulse_##ID(const LaunchDims& d, int n, const MbPhysics& p, float* state, const int* link,     \
+                                  const float* point, const float* impulse) {                                         \
+    k_apply_impulse_##ID<<<d.grid, d.threads, d.smem, d.stream>>>(n, p, state, link, point, impulse);                 \
+  }                                                                                                                   \
   extern const MbKindOps mb_kind_##ID = {ENV_ID, VARIANT, ENV::OBS, ENV::ACT, ENV::REC_STRIDE, ENV::Model::NJ,       \
                                          WARPS, ENV::INFO_FIELD, sizeof(typename ENV::Mem),                          \
                                          ENV::template default_physics<mb200_physics>, ENV::fix_physics, ENV::PARAMS, \
                                          prepare_##ID,                                                               \
                                          launch_step_##ID, launch_reset_##ID, launch_physics_##ID,                    \
-                                         launch_debug_##ID};
+                                         launch_debug_##ID, launch_impulse_##ID};

@@ -283,6 +283,46 @@ class Walker3DCustomVecEnv:
         _lib.check(self._L.mb200_inverse_dynamics(self._h, _ptr(acc), _ptr(tau), self._stream()))
         return tau
 
+    # ---- pushes (mb200_apply_impulse)
+    def link_index(self, name: str) -> int:
+        """The link index ``apply_impulse`` takes for the model link ``name``: -1 for the base, else the dof of the
+        link's movable frame, a fixed link folded into its nearest movable ancestor.  KeyError for unknown names."""
+        t = self.table
+        if name == t["base"]["name"]:
+            return -1
+        if name not in t["link_names"]:
+            raise KeyError("%s has no link %r" % (self.model, name))
+        k = t["link_names"].index(name)
+        while k >= 0 and t["dof_of_link"][k] < 0:
+            k = t["parent"][k]
+        return -1 if k < 0 else int(t["dof_of_link"][k])
+
+    def apply_impulse(self, impulse, link=-1, point=None):
+        """Push every env between two steps: the linear impulse ``impulse`` (N s, world frame, [N, 3] or [3]) at the
+        world point ``point`` ([N, 3] or [3]) rigidly attached to ``link`` (an int or an int tensor [N]; -1 = the base,
+        else see ``link_index``).  The generalised velocity changes by M(q)^-1 J^T impulse (clamped to max_coord_vel);
+        positions, the record and the RNG streams are untouched, and so is every env whose link is outside [-1, NJ)
+        (e.g. -2 masks an env out) or whose impulse is zero or non-finite.  ``point=None`` means the base COM and needs
+        ``link=-1``.  The observation already returned is the pre-push one; the next ``step`` sees the pushed state.
+        CassieEnv keeps its loop closures closed; the planar walkers ignore the y components of impulse and point."""
+        n, dev, nj = self.num_envs, self.device, self.nu - 6
+        scalar_link = isinstance(link, (int, np.integer))
+        if scalar_link:
+            link = int(link)
+            if not -1 <= link < nj:
+                raise ValueError("link %d outside [-1, %d)" % (link, nj))
+            links = torch.full((n,), link, dtype=torch.int32, device=dev)
+        else:
+            links = torch.as_tensor(link).to(device=dev, dtype=torch.int32).expand(n).contiguous()
+        if point is None:
+            if not (scalar_link and link == -1):
+                raise ValueError("point=None (the base COM) needs link=-1")
+            pts = self.get_state()[:, 0:3].contiguous()
+        else:
+            pts = torch.as_tensor(point).to(device=dev, dtype=torch.float32).expand(n, 3).contiguous()
+        imp = torch.as_tensor(impulse).to(device=dev, dtype=torch.float32).expand(n, 3).contiguous()
+        _lib.check(self._L.mb200_apply_impulse(self._h, _ptr(links), _ptr(pts), _ptr(imp), self._stream()))
+
     # ---- trainer-facing extras (env_base.py:103-118, env_locomotion.py:76-77,224-282)
     eval_mode = False  # env_locomotion.py:52
 
@@ -561,6 +601,15 @@ class Walker3DCustomEnv:
 
     def get_mirror_indices(self):
         return self.vec.get_mirror_indices()
+
+    def apply_impulse(self, impulse, link=-1, point=None):
+        """Push the robot before the next ``step``: ``impulse`` (N s, world frame, 3 values) at the world ``point``
+        on ``link`` (see ``Walker3DCustomVecEnv.apply_impulse``; ``link_index`` maps link names)."""
+        pt = None if point is None else np.asarray(point, dtype=np.float32).reshape(3)
+        self.vec.apply_impulse(np.asarray(impulse, dtype=np.float32).reshape(3), link=link, point=pt)
+
+    def link_index(self, name):
+        return self.vec.link_index(name)
 
     def close(self):
         self.vec.close()
