@@ -167,6 +167,36 @@ int mb200_inverse_dynamics(mb200_env* env, const float* acc_dev, float* tau_dev,
 int mb200_apply_impulse(mb200_env* env, const int* link_dev, const float* point_dev, const float* impulse_dev,
                         void* stream);
 
+/* Camera images (pybullet.getCameraImage(width, height, viewMatrix, projectionMatrix) for a batch): for each of `count`
+ * cameras, env env_ids_dev[i] (device memory, [count]; NULL = envs 0..count-1) in its current state -- the state the
+ * last reset / step / set_state / apply_impulse left, i.e. after an auto-reset the first state of the new episode.
+ * An id outside [0, n_envs) gives a blank frame (sky colour, depth = far, seg = -1).
+ *   view_dev, proj_dev: [count][16] float32, column-major OpenGL 4x4 matrices exactly as pybullet.computeViewMatrix*
+ *     and computeProjectionMatrixFOV return them (the same camera can be passed to both).  proj * view is inverted in
+ *     double precision once per camera; a singular or non-finite product gives a blank frame with depth NaN.
+ *   The ray of pixel (row r, column c) runs through NDC x = 2 (c + 0.5) / W - 1, y = 1 - 2 (r + 0.5) / H from the near
+ *     plane to the far plane; row 0 is the top row, as in getCameraImage.  1 <= width, height <= 2048, count >= 1.
+ * Outputs (device memory; any may be NULL, it is then not written):
+ *   rgb_dev   [count][H][W][3] uint8;
+ *   depth_dev [count][H][W] float32: eye-space distance along the view axis in metres (far where nothing is hit).
+ *     Not PyBullet's nonlinear depth buffer: that is  buf = far (depth - near) / (depth (far - near)).
+ *   seg_dev   [count][H][W] int32: -1 sky; 0 ground, 10 + k plank box k (k = 2 p base / 2 p + 1 cover of plank p, the
+ *     Pillar stones likewise), 20 + k bar k (the partner codes of mb200_step_physics_points); 30 the walk target;
+ *     100 + link for a robot link, link as mb200_apply_impulse and the contact list index it (99 = the base, fixed
+ *     links folded into their movable ancestor).
+ * Scene: the collision geometry only (no visual meshes): the robot's spheres, capsules and boxes; CassieEnv-v0's link
+ * hulls as convex polytopes (its hull-vertex contact spheres are not drawn, so a Cassie link without a hull, e.g. the
+ * pelvis, is invisible); the ground plane where physics.has_ground is set; the Stepper / Mike planks as the base and
+ * cover boxes (or the Pillar cylinders) and Monkey3D's four bars, as the collision pass stages them; for the
+ * Walker3DCustomEnv template (Walker3D, Child3D, Walker2D, Crab2D) the walk target as a sphere of radius 0.2 m (a
+ * constant of this library).  Shading is flat and deterministic: one colour per class, a 1 m checkerboard on the
+ * ground, Lambert shading from one fixed directional light plus ambient; no shadows, no anti-aliasing.
+ * Rendering reads the state and the record and writes only its outputs (state, record, RNG streams, warm-start impulses,
+ * statistics and observations are untouched); asynchronous on `stream`.  The handle owns the scene scratch buffer: one
+ * handle's renders on different streams must not overlap. */
+int mb200_render(mb200_env* env, const int* env_ids_dev, int count, const float* view_dev, const float* proj_dev,
+                 int width, int height, uint8_t* rgb_dev, float* depth_dev, int32_t* seg_dev, void* stream);
+
 /* EnvBase.set_env_params analogue (env_base.py:103-106): "eval_mode" (Walker3DCustomEnv, env_locomotion.py:76-77),
  * "curriculum" 0..9 (Walker3DStepperEnv, env_locomotion.py:362-369; takes effect at the next reset like the
  * reference, whose terrain / gain / terminal height are read in reset() and step()), "random_reward" 0 / 1

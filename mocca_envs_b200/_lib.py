@@ -27,7 +27,7 @@ SYMBOLS = [
     "mb200_contact_point_width", "mb200_warm_width", "mb200_get_warm", "mb200_set_warm",
     "mb200_step", "mb200_step_host", "mb200_get_state", "mb200_set_state", "mb200_get_record", "mb200_set_record",
     "mb200_rng_words", "mb200_get_rng", "mb200_set_rng", "mb200_step_physics", "mb200_mass_matrix", "mb200_inverse_dynamics",
-    "mb200_apply_impulse", "mb200_set_param",
+    "mb200_apply_impulse", "mb200_render", "mb200_set_param",
     "mb200_set_param_array", "mb200_record_stride", "mb200_stats",
     "mb200_launch_count", "mb200_measure_fp32_peak", "mb200_last_error",
 ]
@@ -122,6 +122,7 @@ def lib():
         L.mb200_set_rng.argtypes = [vp, vp]
         L.mb200_inverse_dynamics.argtypes = [vp, vp, vp, vp]
         L.mb200_apply_impulse.argtypes = [vp, vp, vp, vp, vp]
+        L.mb200_render.argtypes = [vp, vp, ip, vp, vp, ip, ip, vp, vp, vp, vp]
         L.mb200_set_param.argtypes = [vp, C.c_char_p, C.c_float]
         L.mb200_set_param_array.argtypes = [vp, C.c_char_p, vp, ip]
         L.mb200_record_stride.argtypes = [vp]

@@ -11,6 +11,8 @@ Kernel-side representation (all constant, derived at q = 0):
   per link and non-linear in |v| (SURVEY App. G).
 * points              : contact candidates -- sphere centres and both capsule end-sphere centres.
 * generalised coordinates u = [omega_world, v_baseCOM_world, qd] (PyBullet/btMultiBody order), NU = 6 + NJ.
+* render geoms         : the collision geometry as mb200_render draws it (sphere, capsule, box in the owner joint
+  frame) and the face planes of the mesh hulls; read by the render kernels only.
 """
 from __future__ import annotations
 
@@ -180,6 +182,23 @@ def reduce_table(t: dict) -> dict:
                            pack=ha | (hb << 8), thresh=th, mu=A["friction"] * B["friction"], own_a=A["owner"],
                            own_b=B["owner"], feet=feet))
         assert A["owner"] != B["owner"]
+    # render geoms (mb200_render): every sphere / capsule / box in its owner joint frame.  A model with mesh hulls
+    # (Cassie) is drawn as its hulls; its geoms are the hull-vertex contact spheres and are not drawn.
+    rgeoms = []
+    for g in ([] if hulls else t["geoms"]):
+        link = g["link"]
+        oj = owner_joint(link) if link >= 0 else -1
+        Ro, oo = frame(oj)
+        loc = lambda v: Ro.T @ (pl[link + 1] + Rl[link + 1] @ np.array(v) - oo)
+        if g["type"] == GEOM_BOX:
+            rgeoms.append(dict(type=2, owner=oj, a=loc(g["pos"]), b=loc(g["pos"]), r=0.0,
+                               rot=(Ro.T @ Rl[link + 1] @ quat_to_mat(g["quat"])).reshape(9), half=g["size"][:3]))
+        elif g["type"] in (GEOM_SPHERE, GEOM_CAPSULE):
+            p1 = g["p0"] if g["type"] == GEOM_SPHERE else g["p1"]
+            rgeoms.append(dict(type=0 if g["type"] == GEOM_SPHERE else 1, owner=oj, a=loc(g["p0"]), b=loc(p1),
+                               r=g["size"][0], rot=np.eye(3).reshape(9), half=[0.0, 0.0, 0.0]))
+    for h in hulls:
+        h["planes"] = hull_planes(h["verts"])
     # ancestor chains (root -> self) packed 5 bits per entry, and the compact (chain-ordered) factor layout:
     # row i of L stores only its support [base block | ancestors root->parent | diagonal]
     chains = []
@@ -212,7 +231,7 @@ def reduce_table(t: dict) -> dict:
         extras = dict(ordered=t["ordered_dofs"], pd_dof=[t["ordered_dofs"][k] for k in pd], pd_ordered=pd,
                       pd_kp=t["pd_kp"], pd_kd=t["pd_kd"], npowered=len(t["powered_joint_inds"]))
     return dict(name=t["name"], nj=nj, nb=nb, nu=6 + nj, npt=len(points), nlevel=max(jlevel) + 1,
-                xboxes=xboxes, palm_body=palm_body, p2p=p2p, extras=extras, spairs=spairs, hulls=hulls,
+                xboxes=xboxes, palm_body=palm_body, rgeoms=rgeoms, p2p=p2p, extras=extras, spairs=spairs, hulls=hulls,
                 hull_margin=t.get("hull_margin", 0.0),
                 jparent=jparent, joff=joff, jrot=jrot, jaxis=jaxis, jlevel=jlevel, janc=janc,
                 lower=t["lower"], upper=t["upper"], gain=t["gain"], damping=t["damping"], armature=t["armature"],
@@ -221,6 +240,20 @@ def reduce_table(t: dict) -> dict:
                 right=t["right_joint_indices"], left=t["left_joint_indices"], neg=t["negation_joint_indices"],
                 jdepth=jdepth, chainpack=chainpack, rowlen=rowlen, rowoff=rowoff, rowmask_rt=rowmask_rt,
                 lsize=sum(rowlen), maxsup=max(rowlen))
+
+
+def hull_planes(verts) -> np.ndarray:
+    """Face planes [k][4] = (n, d), |n| = 1, of the convex hull of `verts`: n . x <= d inside.  Coplanar facets of
+    scipy's triangulation are merged, so each plane is one face."""
+    from scipy.spatial import ConvexHull
+
+    V = np.asarray(verts, dtype=np.float64)
+    planes = []
+    for eq in ConvexHull(V).equations:  # n . x + off <= 0 inside, |n| = 1
+        n, d = eq[:3], -eq[3]
+        if not any(np.abs(n - p[:3]).max() < 1e-9 and abs(d - p[3]) < 1e-9 for p in planes):
+            planes.append(np.concatenate([n, [d]]))
+    return np.array(planes)
 
 
 def _f(v) -> str:
@@ -423,6 +456,23 @@ def emit_header(t: dict, prefix: str) -> str:
     out.append(_iarr(P + "_right", r["right"]))
     out.append(_iarr(P + "_left", r["left"]))
     out.append(_iarr(P + "_neg", r["neg"]))
+    # render tables (mb200_render only): geoms in their owner joint frames, the hulls' face planes (n, d) in the same
+    # frames, hull h owning planes [hpl_off[h], hpl_off[h + 1]).  Constant memory, declared behind every other table:
+    # the physics kernels' global-table addresses (constant bank 4) and constant tables keep their slots.
+    rg = r["rgeoms"] or [dict(type=-1, owner=-1, a=[0, 0, 0], b=[0, 0, 0], r=0, rot=np.eye(3).reshape(9), half=[0, 0, 0])]
+    out.append(_iarr(P + "_rg_type", [g["type"] for g in rg]).replace("MB_TABLE", "MB_CTABLE"))
+    out.append(_iarr(P + "_rg_owner", [g["owner"] for g in rg]).replace("MB_TABLE", "MB_CTABLE"))
+    out.append(_farr(P + "_rg_a", [g["a"] for g in rg]).replace("MB_TABLE", "MB_CTABLE"))
+    out.append(_farr(P + "_rg_b", [g["b"] for g in rg]).replace("MB_TABLE", "MB_CTABLE"))
+    out.append(_farr(P + "_rg_r", [g["r"] for g in rg]).replace("MB_TABLE", "MB_CTABLE"))
+    out.append(_farr(P + "_rg_rot", [g["rot"] for g in rg]).replace("MB_TABLE", "MB_CTABLE"))
+    out.append(_farr(P + "_rg_half", [g["half"] for g in rg]).replace("MB_TABLE", "MB_CTABLE"))
+    hpl = [p for h in r["hulls"] for p in h["planes"]] or [[0.0, 0.0, 1.0, 0.0]]
+    hoff = [0]
+    for h in r["hulls"]:
+        hoff.append(hoff[-1] + len(h["planes"]))
+    out.append(_iarr(P + "_hpl_off", hoff).replace("MB_TABLE", "MB_CTABLE"))
+    out.append(_farr(P + "_hpl", hpl).replace("MB_TABLE", "MB_CTABLE"))
     # support of row i of the mass matrix / its L^T L factor (columns j < i): base block + ancestors
     rowmask = []
     for i in range(r["nu"]):
@@ -441,6 +491,9 @@ def emit_header(t: dict, prefix: str) -> str:
                   r["lsize"], r["maxsup"], len(r["xboxes"]), len(r["p2p"]), len(ex.get("ordered", [])),
                   len(ex.get("pd_dof", [])), ex.get("npowered", 0), len(sp),
                   len(r["hulls"]), int(bool(r["hulls"]) and bool(sp))))
+    out.append("  enum { NRG = %d, NHPL = %d };  // render geoms, hull face planes (mb200_render)\n"
+               % (len(r["rgeoms"]), len(hpl) if r["hulls"] else 0))
+    out.append("  MB_HD static const float* hpl() { return &%s_hpl[0][0]; }\n" % P)
     out.append("  MB_HD static float hull_margin() { return %s; }\n" % _f(r["hull_margin"]))
     out.append("  MB_HD static int hown(int i) { return %s_hown[i]; }\n" % P)
     out.append("  MB_HD static float hcen(int i, int k) { return %s_hcen[i][k]; }\n" % P)
@@ -475,13 +528,14 @@ def emit_header(t: dict, prefix: str) -> str:
                        ("bowner", "int"), ("powner", "int"), ("pfoot", "int"), ("pid", "int"), ("foot_body", "int"),
                        ("palm_body", "int"), ("xowner", "int"), ("xfoot", "int"), ("xpid", "int"),
                        ("lc_owner", "int"), ("ordered", "int"), ("pd_dof", "int"), ("pd_ordered", "int"),
-                       ("right", "int"), ("left", "int"), ("neg", "int"), ("sp_pack", "unsigned"), ("sp_own", "int")]:
+                       ("right", "int"), ("left", "int"), ("neg", "int"), ("sp_pack", "unsigned"), ("sp_own", "int"),
+                       ("rg_type", "int"), ("rg_owner", "int"), ("hpl_off", "int")]:
         out.append("  MB_HD static %s %s(int i) { return %s_%s[i]; }\n" % (ctype, fld, P, fld))
     out.append("  MB_HD static double base_angles(int i) { return %s_base_angles[i]; }\n" % P)
     for fld in ["lower", "upper", "weight", "gain", "damping", "armature", "bmass", "pradius", "pfriction", "pthresh",
-                "xfriction", "xthresh", "lc_maximp", "pd_kp", "pd_kd", "sp_thresh", "sp_mu", "sp_reach"]:
+                "xfriction", "xthresh", "lc_maximp", "pd_kp", "pd_kd", "sp_thresh", "sp_mu", "sp_reach", "rg_r"]:
         out.append("  MB_HD static float %s(int i) { return %s_%s[i]; }\n" % (fld, P, fld))
-    for fld in ["bcom", "binertia", "ppos", "xpos", "xrot", "xhalf", "lc_pos"]:
+    for fld in ["bcom", "binertia", "ppos", "xpos", "xrot", "xhalf", "lc_pos", "rg_a", "rg_b", "rg_rot", "rg_half"]:
         out.append("  MB_HD static float %s(int i, int k) { return %s_%s[i][k]; }\n" % (fld, P, fld))
     out.append("  MB_HD static float base_x() { return %s; }\n" % _f(r["base_position"][0]))
     out.append("  MB_HD static float base_y() { return %s; }\n" % _f(r["base_position"][1]))

@@ -77,6 +77,8 @@ struct mb200_env {
   int* hist;       // [2][256] step t counts into hist[t & 1]; the scatter kernel zeroes the other half
   int* cursor;     // [2][256] scatter cursors, same double buffering
   int sort_every;  // 0 = never re-sort (identity order), otherwise after every step
+  float* render_scene;  // [render_cap][MB_RMAX][MB_RSTRIDE] primitive lists of mb200_render's scene pass
+  int render_cap;       // cameras the scene buffer holds
   long long steps;
   long long launches;
   size_t smem;
@@ -274,6 +276,7 @@ void mb200_destroy(mb200_env* e) {
   if (e->host_done) cudaEventDestroy(e->host_done);
   cudaFree(e->dummy_obs); cudaFree(e->dummy_rew); cudaFree(e->dummy_flag); cudaFree(e->dummy_stats);
   cudaFree(e->order); cudaFree(e->key); cudaFree(e->hist); cudaFree(e->cursor);
+  cudaFree(e->render_scene);
   delete e;
 }
 
@@ -598,6 +601,61 @@ int mb200_apply_impulse(mb200_env* e, const int* link_dev, const float* point_de
   const LaunchDims d = {grid_for(e), e->warps * 32, e->smem, (cudaStream_t)stream};
   e->ops->impulse(d, e->n, e->phys, e->state, link_dev, point_dev, impulse_dev);
   e->launches++;
+  CUDA_OK(cudaGetLastError());
+  return 0;
+}
+
+// mb200_render, pass 2: one CTA per (camera, 16 x 16 pixel tile), one thread per pixel.  The CTA stages the camera's
+// primitive list in shared memory and inverts its proj * view once (double); every thread then casts its pixel's ray
+// (mb_render_pixel) and stores RGB, depth and segmentation.
+#define MB_RENDER_TILE 16
+__global__ void __launch_bounds__(MB_RENDER_TILE* MB_RENDER_TILE)
+    k_render_rays(int nprim, const float* scene, const float* view, const float* proj, int W, int H, uint8_t* rgb,
+                  float* depth, int* seg) {
+  __shared__ __align__(16) float prims[MB_RMAX * MB_RSTRIDE];
+  __shared__ MbCamera cam;
+  const int c = blockIdx.x, tid = threadIdx.x;
+  const int tiles_x = (W + MB_RENDER_TILE - 1) / MB_RENDER_TILE;
+  const int tx = blockIdx.y % tiles_x, ty = blockIdx.y / tiles_x;
+  const float* src = scene + (size_t)c * MB_RMAX * MB_RSTRIDE;
+  for (int i = tid; i < nprim * MB_RSTRIDE; i += blockDim.x) prims[i] = src[i];
+  if (tid == 0) mb_render_camera(view + 16 * (size_t)c, proj + 16 * (size_t)c, &cam);
+  __syncthreads();
+  const int col = tx * MB_RENDER_TILE + tid % MB_RENDER_TILE, row = ty * MB_RENDER_TILE + tid / MB_RENDER_TILE;
+  if (col >= W || row >= H) return;
+  const size_t px = ((size_t)c * H + row) * W + col;
+  uint8_t p3[3];
+  float dp;
+  int sg;
+  mb_render_pixel(cam, prims, nprim, W, H, row, col, rgb ? p3 : nullptr, &dp, &sg);
+  if (rgb) { rgb[3 * px] = p3[0]; rgb[3 * px + 1] = p3[1]; rgb[3 * px + 2] = p3[2]; }
+  if (depth) depth[px] = dp;
+  if (seg) seg[px] = sg;
+}
+
+int mb200_render(mb200_env* e, const int* env_ids_dev, int count, const float* view_dev, const float* proj_dev,
+                 int width, int height, uint8_t* rgb_dev, float* depth_dev, int32_t* seg_dev, void* stream) {
+  if (!e) return fail("mb200_render: NULL argument");
+  if (count < 1) return fail("mb200_render: count must be >= 1, got " + std::to_string(count));
+  if (width < 1 || width > MB_RENDER_MAXDIM || height < 1 || height > MB_RENDER_MAXDIM)
+    return fail("mb200_render: width and height must be in [1, " + std::to_string(MB_RENDER_MAXDIM) + "], got " +
+                std::to_string(width) + " x " + std::to_string(height));
+  if (!view_dev || !proj_dev) return fail("mb200_render: NULL view or projection matrices");
+  CUDA_OK(cudaSetDevice(e->device));
+  if (count > e->render_cap) {
+    cudaFree(e->render_scene);
+    e->render_scene = nullptr;
+    e->render_cap = 0;
+    CUDA_OK(cudaMalloc(&e->render_scene, (size_t)count * MB_RMAX * MB_RSTRIDE * sizeof(float)));
+    e->render_cap = count;
+  }
+  const cudaStream_t st = (cudaStream_t)stream;
+  const LaunchDims d = {(count + e->warps - 1) / e->warps, e->warps * 32, e->smem, st};
+  e->ops->render(d, e->n, count, e->phys, e->state, e->rec, env_ids_dev, e->render_scene);
+  const int tiles = ((width + MB_RENDER_TILE - 1) / MB_RENDER_TILE) * ((height + MB_RENDER_TILE - 1) / MB_RENDER_TILE);
+  k_render_rays<<<dim3(count, tiles), MB_RENDER_TILE * MB_RENDER_TILE, 0, st>>>(
+      e->ops->render_nprim, e->render_scene, view_dev, proj_dev, width, height, rgb_dev, depth_dev, seg_dev);
+  e->launches += 2;
   CUDA_OK(cudaGetLastError());
   return 0;
 }

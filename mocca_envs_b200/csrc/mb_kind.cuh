@@ -22,6 +22,7 @@
 
 #include "../../include/mocca_b200.h"
 #include "mb_env.cuh"
+#include "mb_render.cuh"
 
 struct StepArgs {
   int n;
@@ -78,6 +79,9 @@ struct MbKindOps {
   void (*debug)(const LaunchDims&, int n, const MbPhysics&, const float* state, int mode, const float* acc, float* out);
   void (*impulse)(const LaunchDims&, int n, const MbPhysics&, float* state, const int* link, const float* point,
                   const float* impulse);
+  int render_nprim;  // primitives per camera of the render scene pass (MbRenderLayout<Env>::NPRIM <= MB_RMAX)
+  void (*render)(const LaunchDims&, int n, int count, const MbPhysics&, const float* state, const float* rec,
+                 const int* ids, float* scene);
 };
 
 template <class Env, bool HOST>
@@ -212,8 +216,27 @@ __device__ __forceinline__ void impulse_body(int n, const MbPhysics& phys, float
                         impulse + 3 * (size_t)env);
 }
 
-// One env kind: step (device / host-buffer instantiations), reset, physics-only, debug and impulse kernels + its
-// MbKindOps.
+// mb200_render, pass 1: camera `cam` gets the world-space primitive list of env ids[cam] (mb_render_scene); an id
+// outside the batch gets an empty list (a blank frame).  No CTA barrier on this path.
+template <class Env>
+__device__ __forceinline__ void render_scene_body(int n, int count, const MbPhysics& phys, const float* state,
+                                                  const float* rec, const int* ids, float* scene) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  const int warp = threadIdx.x >> 5;
+  const int cam = blockIdx.x * MB_WARPS + warp;
+  if (cam >= count) return;
+  const int env = ids ? ids[cam] : cam;
+  float* out = scene + (size_t)cam * MB_RMAX * MB_RSTRIDE;
+  if (env < 0 || env >= n) {
+    mb_render_blank(out, MbRenderLayout<Env>::NPRIM);
+    return;
+  }
+  typename Env::Mem& S = reinterpret_cast<typename Env::Mem*>(smem_raw)[warp];
+  mb_render_scene<Env>(S, phys, state + (size_t)env * MB_STATE_STRIDE, rec + (size_t)env * Env::REC_STRIDE, out);
+}
+
+// One env kind: step (device / host-buffer instantiations), reset, physics-only, debug, impulse and render-scene
+// kernels + its MbKindOps.
 #define MB_DEFINE_KIND(ID, ENV_ID, VARIANT, ENV, WARPS)                                                               \
   __global__ void __launch_bounds__(WARPS * 32, MB_MINBLOCKS) k_step_##ID(StepArgs a) { step_body<ENV, false>(a); }  \
   __global__ void __launch_bounds__(WARPS * 32, MB_MINBLOCKS) k_step_##ID##_host(StepArgs a) {                       \
@@ -238,6 +261,11 @@ __device__ __forceinline__ void impulse_body(int n, const MbPhysics& phys, float
                            const float* impulse) {                                                                    \
     impulse_body<ENV>(n, phys, state, link, point, impulse);                                                          \
   }                                                                                                                   \
+  __global__ void __launch_bounds__(MB_WARPS_MAX * 32)                                                                \
+      k_render_scene_##ID(int n, int count, MbPhysics phys, const float* state, const float* rec, const int* ids,    \
+                          float* scene) {                                                                             \
+    render_scene_body<ENV>(n, count, phys, state, rec, ids, scene);                                                   \
+  }                                                                                                                   \
   static cudaError_t prepare_##ID(void) {                                                                             \
     const int bytes = (int)(sizeof(typename ENV::Mem) * WARPS);                                                \
     const cudaFuncAttribute at = cudaFuncAttributeMaxDynamicSharedMemorySize;                                         \
@@ -247,7 +275,8 @@ __device__ __forceinline__ void impulse_body(int n, const MbPhysics& phys, float
     if ((e = cudaFuncSetAttribute(k_reset_##ID, at, bytes)) != cudaSuccess) return e;                                 \
     if ((e = cudaFuncSetAttribute(k_step_physics_##ID, at, bytes)) != cudaSuccess) return e;                          \
     if ((e = cudaFuncSetAttribute(k_dynamics_debug_##ID, at, bytes)) != cudaSuccess) return e;                       \
-    return cudaFuncSetAttribute(k_apply_impulse_##ID, at, bytes);                                                     \
+    if ((e = cudaFuncSetAttribute(k_apply_impulse_##ID, at, bytes)) != cudaSuccess) return e;                         \
+    return cudaFuncSetAttribute(k_render_scene_##ID, at, bytes);                                                      \
   }                                                                                                                   \
   static void launch_step_##ID(const StepArgs& a, bool host, const LaunchDims& d) {                                   \
     if (host) k_step_##ID##_host<<<d.grid, d.threads, d.smem, d.stream>>>(a);                                         \
@@ -271,9 +300,14 @@ __device__ __forceinline__ void impulse_body(int n, const MbPhysics& phys, float
                                   const float* point, const float* impulse) {                                         \
     k_apply_impulse_##ID<<<d.grid, d.threads, d.smem, d.stream>>>(n, p, state, link, point, impulse);                 \
   }                                                                                                                   \
+  static void launch_render_##ID(const LaunchDims& d, int n, int count, const MbPhysics& p, const float* state,       \
+                                 const float* rec, const int* ids, float* scene) {                                    \
+    k_render_scene_##ID<<<d.grid, d.threads, d.smem, d.stream>>>(n, count, p, state, rec, ids, scene);                \
+  }                                                                                                                   \
   extern const MbKindOps mb_kind_##ID = {ENV_ID, VARIANT, ENV::OBS, ENV::ACT, ENV::REC_STRIDE, ENV::Model::NJ,       \
                                          WARPS, ENV::INFO_FIELD, sizeof(typename ENV::Mem),                          \
                                          ENV::template default_physics<mb200_physics>, ENV::fix_physics, ENV::PARAMS, \
                                          prepare_##ID,                                                               \
                                          launch_step_##ID, launch_reset_##ID, launch_physics_##ID,                    \
-                                         launch_debug_##ID, launch_impulse_##ID};
+                                         launch_debug_##ID, launch_impulse_##ID,                                     \
+                                         MbRenderLayout<ENV>::NPRIM, launch_render_##ID};

@@ -53,6 +53,48 @@ def _ptr(t):
     return None if t is None else C.c_void_p(t.data_ptr())
 
 
+# The tracking camera of VecEnv.render / render(mode="rgb_array") when no camera is given: PyBullet's yaw / pitch /
+# distance convention about the env's base position (yaw 0 = looking along +y, i.e. at the x-z plane of the walkers)
+TRACKING_CAMERA = dict(distance=3.0, yaw=0.0, pitch=-20.0, fov=60.0, near=0.01, far=100.0)
+RENDER_OUTPUTS = ("rgb", "depth", "seg")
+
+
+def camera_matrices(target, distance, yaw, pitch, fov=60.0, aspect=1.0, near=0.01, far=100.0):
+    """(view, proj), float32 torch tensors [m, 16]: column-major OpenGL matrices in the layout of
+    ``pybullet.computeViewMatrixFromYawPitchRoll(target, distance, yaw, pitch, 0, upAxisIndex=2)`` and
+    ``pybullet.computeProjectionMatrixFOV(fov, aspect, near, far)``, for ``mb200_render`` / ``VecEnv.render``.
+
+    ``target`` is [3] or [m, 3] (a tensor keeps its device).  Angles are in degrees, z is up: the eye sits at
+    ``target + distance * (cos(pitch) sin(yaw), -cos(pitch) cos(yaw), -sin(pitch))`` (so a negative pitch looks down),
+    looks at the target, and its up vector is ``(sin(pitch) sin(yaw), -sin(pitch) cos(yaw), cos(pitch))``.  PyBullet is
+    not a dependency here, so only these geometric properties are checked, not the matrices against PyBullet's."""
+    t = torch.as_tensor(target, dtype=torch.float64)
+    t = t.reshape(-1, 3)
+    m, dev = t.shape[0], t.device
+    y, p = np.deg2rad(float(yaw)), np.deg2rad(float(pitch))
+    off = torch.tensor([np.cos(p) * np.sin(y), -np.cos(p) * np.cos(y), -np.sin(p)], dtype=torch.float64, device=dev)
+    up = torch.tensor([np.sin(p) * np.sin(y), -np.sin(p) * np.cos(y), np.cos(p)], dtype=torch.float64, device=dev)
+    eye = t + float(distance) * off
+    f = torch.nn.functional.normalize(t - eye, dim=1)
+    sv = torch.nn.functional.normalize(torch.cross(f, up.expand(m, 3), dim=1), dim=1)
+    u = torch.cross(sv, f, dim=1)
+    view = torch.zeros(m, 16, dtype=torch.float64, device=dev)
+    view[:, [0, 4, 8]] = sv
+    view[:, [1, 5, 9]] = u
+    view[:, [2, 6, 10]] = -f
+    view[:, 12] = -(sv * eye).sum(1)
+    view[:, 13] = -(u * eye).sum(1)
+    view[:, 14] = (f * eye).sum(1)
+    view[:, 15] = 1.0
+    ys = 1.0 / np.tan(np.deg2rad(float(fov)) / 2)
+    proj = torch.zeros(m, 16, dtype=torch.float64, device=dev)
+    proj[:, 0], proj[:, 5] = ys / float(aspect), ys
+    proj[:, 10] = (far + near) / (near - far)
+    proj[:, 11] = -1.0
+    proj[:, 14] = 2.0 * far * near / (near - far)
+    return view.float(), proj.float()
+
+
 def _unsupported(message=None):
     """A trainer-facing method the reference env does not have: it raises AttributeError(message), or does nothing
     when there is no message."""
@@ -323,6 +365,45 @@ class Walker3DCustomVecEnv:
         imp = torch.as_tensor(impulse).to(device=dev, dtype=torch.float32).expand(n, 3).contiguous()
         _lib.check(self._L.mb200_apply_impulse(self._h, _ptr(links), _ptr(pts), _ptr(imp), self._stream()))
 
+    # ---- camera images (mb200_render)
+    def render(self, env_ids=None, width=64, height=64, view=None, proj=None, outputs=RENDER_OUTPUTS):
+        """Camera images of envs ``env_ids`` (None = every env, else an int tensor / sequence, any order, repeats
+        allowed, an id outside the batch gives a blank frame) in their current state, by ray casting the collision
+        geometry on the device: a dict with the requested ``outputs`` of "rgb" ([m, H, W, 3] uint8), "depth"
+        ([m, H, W] float32, eye-space distance along the view axis, ``far`` where nothing is hit) and "seg" ([m, H, W]
+        int32: -1 sky, 0 ground, 10 + k plank box, 20 + k bar, 30 walk target, 100 + link for a robot link).
+        ``view`` / ``proj`` are [16] or [m, 16] column-major OpenGL matrices as ``camera_matrices`` and PyBullet build
+        them; without them a tracking camera (``TRACKING_CAMERA``) looks at each env's base position.  The envs'
+        state, record and RNG streams are untouched.  See include/mocca_b200.h: mb200_render."""
+        unknown = set(outputs) - set(RENDER_OUTPUTS)
+        if unknown:
+            raise ValueError("unknown render outputs %s: choose from %s" % (sorted(unknown), RENDER_OUTPUTS))
+        dev = self.device
+        ids = None if env_ids is None else torch.as_tensor(env_ids).to(device=dev, dtype=torch.int32).reshape(-1)
+        m = self.num_envs if ids is None else int(ids.numel())
+        W, H = int(width), int(height)
+        if view is None or proj is None:
+            st = self.get_state()[:, 0:3]
+            if ids is not None:
+                ok = (ids >= 0) & (ids < self.num_envs)
+                st = torch.where(ok[:, None], st[ids.clamp(0, self.num_envs - 1).long()], torch.zeros_like(st[:1]))
+            v, p = camera_matrices(st, aspect=W / H if W > 0 and H > 0 else 1.0, **TRACKING_CAMERA)
+            view = v if view is None else view
+            proj = p if proj is None else proj
+        view = torch.as_tensor(view).to(device=dev, dtype=torch.float32).expand(m, 16).contiguous()
+        proj = torch.as_tensor(proj).to(device=dev, dtype=torch.float32).expand(m, 16).contiguous()
+        kw = dict(device=dev)
+        out = {}
+        if "rgb" in outputs:
+            out["rgb"] = torch.empty(m, max(H, 0), max(W, 0), 3, dtype=torch.uint8, **kw)
+        if "depth" in outputs:
+            out["depth"] = torch.empty(m, max(H, 0), max(W, 0), dtype=torch.float32, **kw)
+        if "seg" in outputs:
+            out["seg"] = torch.empty(m, max(H, 0), max(W, 0), dtype=torch.int32, **kw)
+        _lib.check(self._L.mb200_render(self._h, _ptr(ids), m, _ptr(view), _ptr(proj), W, H, _ptr(out.get("rgb")),
+                                        _ptr(out.get("depth")), _ptr(out.get("seg")), self._stream()))
+        return out
+
     # ---- trainer-facing extras (env_base.py:103-118, env_locomotion.py:76-77,224-282)
     eval_mode = False  # env_locomotion.py:52
 
@@ -536,7 +617,7 @@ class CassieVecEnv(Walker3DCustomVecEnv):
 class Walker3DCustomEnv:
     """gym-protocol facade over a 1-env batch; NumPy float64 observations like the reference."""
 
-    metadata = {"render.modes": []}
+    metadata = {"render.modes": ["rgb_array"]}
     vec_class = Walker3DCustomVecEnv
     vec_kwargs = ()  # reference constructor kwargs this env's VecEnv understands
 
@@ -610,6 +691,15 @@ class Walker3DCustomEnv:
 
     def link_index(self, name):
         return self.vec.link_index(name)
+
+    def render(self, mode="rgb_array", width=320, height=240):
+        """An [height, width, 3] uint8 frame of the env from the tracking camera (``VecEnv.render``).  There is no
+        GUI: mode="human" raises NotImplementedError."""
+        if mode == "human":
+            raise NotImplementedError("render(mode='human') needs a GUI; the GPU path renders mode='rgb_array' only")
+        if mode != "rgb_array":
+            raise ValueError("render mode %r: one of %s" % (mode, self.metadata["render.modes"]))
+        return self.vec.render(width=width, height=height, outputs=("rgb",))["rgb"][0].cpu().numpy()
 
     def close(self):
         self.vec.close()
